@@ -128,13 +128,18 @@ def build_tools(force=False):
     return SYNTH_BIN
 
 
+def oracle_available():
+    return os.path.isdir(REFERENCE) or os.path.exists(ORACLE_BIN)
+
+
 def build_oracle(force=False):
-    """Compiles the unmodified reference against the shim. Only possible where /root/reference exists; elsewhere the
-    prebuilt oracle/_ref/arriba (shipped by gpurun) is used as is."""
+    """Compiles the unmodified reference against the shim where its sources are readable; elsewhere a prebuilt
+    oracle/_ref/arriba is used as is. Only recording the reference's results (tests/worldutil.py) and bench.py's
+    CPU baseline run it."""
     if os.path.isdir(REFERENCE):
         _run(["make", "-C", os.path.join(ROOT, "oracle"), "-j8"])
     if not os.path.exists(ORACLE_BIN):
-        raise RuntimeError("oracle/_ref/arriba is missing and /root/reference is not available to build it")
+        raise RuntimeError("oracle/_ref/arriba is missing and the reference sources are not available to build it")
     return ORACLE_BIN
 
 

@@ -141,6 +141,35 @@ REFERENCE_FULL_SIZE = {"cfg2_10M_2x101_50k": {"fragments": 11810114, "seconds": 
                        "cfg3_15M_2x151_75k": {"fragments": 17587876, "seconds": None, "value": None, "cores": 1, "where": "development container: stopped after 3 h 1 min of CPU time inside filter_mismappers, not finished (profiles/r02z/full_size_host_parity.txt)"}}
 
 
+CANDIDATE_COLUMNS = ("gene1", "gene2", "contig1", "contig2", "breakpoint1", "breakpoint2", "direction1", "direction2", "split_reads1", "split_reads2", "discordant_mates",
+                     "filter", "evalue", "confidence", "order")
+DUMP_ROWS = 1 << 18   # 18 arrays (columns and row indexes) of at most 2^18 float64 values: 36 MB, under 64 MB
+
+
+def step_outputs(p):
+    """What a caller of the Pipeline receives after a step: the candidate table (one array per column) and the final label of every fragment."""
+    c = p.candidates()
+    out = {"candidates." + k: c[k] for k in CANDIDATE_COLUMNS}
+    out["fragments.label"] = c["labels"]
+    return out
+
+
+def write_outputs(d, outputs):
+    """DIR/<table>.<column>.npy in float64; a table longer than DUMP_ROWS is sampled at rows chosen by a fixed seed (DIR/<table>.rows.npy)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    rows = {}
+    for name, a in sorted(outputs.items()):
+        table = name.split(".")[0]
+        a = np.asarray(a)
+        if len(a) > DUMP_ROWS:
+            if table not in rows:
+                rows[table] = np.sort(np.random.default_rng(0).choice(len(a), DUMP_ROWS, replace=False))
+                np.save(os.path.join(d, table + ".rows.npy"), rows[table].astype(np.float64))
+            a = a[rows[table]]
+        np.save(os.path.join(d, name + ".npy"), a.astype(np.float64))
+
+
 class QuietStderr:
     """The library prints the reference's per-row warnings on stderr (thousands per step on the synthetic GTF). They go to a log file; the few progress
     lines of this script go to the real stderr."""
@@ -174,7 +203,11 @@ def main():
     ap.add_argument("--mode", choices=["samples", "sharded"], default="sharded",
                     help="N>1: 'sharded' = ONE sample divided over the ranks (strong scaling, NCCL exchanges); 'samples' = one independent sample per GPU (weak scaling, no collective)")
     ap.add_argument("--no-parity", action="store_true", help="skip the md5 comparison of the output files with the reference's")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (candidate table, fragment labels) as DIR/<name>.npy, float64, "
+                                                            "a fixed sample of rows where the table exceeds 64 MB; the inputs are the same from run to run")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     cores = os.cpu_count() or 1
@@ -234,8 +267,8 @@ def main():
     quiet = QuietStderr(os.path.join(outdir, "library_stderr.log")); quiet.__enter__()
     say = (lambda s: quiet.say(s)) if rank == 0 else (lambda s: None)
 
-    def one_step(sharded):
-        """ingest .. fusions.tsv through the public Pipeline API; returns a dict of what the step measured"""
+    def one_step(sharded, capture=False):
+        """ingest .. fusions.tsv through the public Pipeline API; returns a dict of what the step measured (and, with capture, of what it computed)"""
         # one sample divided over the ranks: rank 0 does the host work with all host threads, the others only hold a device context
         p = L.Pipeline(prefix + ".bam", prefix + ".gtf", prefix + ".fa", threads=(threads_all if rank == 0 else 2) if sharded else threads, device=local_rank, output=out_tsv, discarded=out_disc)
         if not sharded or rank == 0:
@@ -278,17 +311,19 @@ def main():
         ev = {n: round(st.event_seconds[i], 2) for i, n in enumerate(L.EV_NAMES) if st.event_seconds[i] >= 0.2}
         say("[bench] step: e2e %.2f s, device %.1f ms, ingest %.2f, annotate %.2f, upload %.2f, output %.2f, events >= 0.2 s: %s" %
             (e2e_s, dev_ms, st.seconds[L.STEP_INGEST], st.seconds[L.STEP_ANNOTATE], st.seconds[L.STEP_UPLOAD], st.output_seconds, ev))
+        outputs = step_outputs(p) if capture and rank == 0 else None   # after the clock stopped
         p.close()
-        return {"n": int(st.n_fragments), "e2e_s": e2e_s, "dev_ms": dev_ms, "st": st, "tm": tm, "d2h": d2h, "n_cand": n_cand, "d2h_parts": d2h_parts, "h2d_parts": h2d_parts}
+        return {"n": int(st.n_fragments), "e2e_s": e2e_s, "dev_ms": dev_ms, "st": st, "tm": tm, "d2h": d2h, "n_cand": n_cand, "d2h_parts": d2h_parts, "h2d_parts": h2d_parts,
+                "outputs": outputs}
 
-    def timed(sharded, warmup, steps):
+    def timed(sharded, warmup, steps, capture=False):
         for _ in range(warmup):
             one_step(sharded)
         if dist:
             dist.barrier()
         torch.cuda.synchronize()
         t_begin = time.perf_counter()
-        results = [one_step(sharded) for _ in range(steps)]
+        results = [one_step(sharded, capture and i == steps - 1) for i in range(steps)]
         torch.cuda.synchronize()
         if dist:
             dist.barrier()
@@ -311,7 +346,7 @@ def main():
         for _ in range(args.warmup):
             one_step(sharded)
         launches1 = lib.arb_kernel_launches()
-        results, e2e_s, dev_ms, wall = timed(sharded, 0, args.steps)
+        results, e2e_s, dev_ms, wall = timed(sharded, 0, args.steps, capture=bool(args.dump_outputs))
     except BaseException:
         import traceback
         quiet.say("bench.py (rank %d): a step failed\n%s" % (rank, traceback.format_exc()))   # on the real stderr, not in the library's log
@@ -319,6 +354,8 @@ def main():
         raise
     launches = lib.arb_kernel_launches() - launches1
     sampler.stop_flag = True; sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, results[-1]["outputs"])
 
     # parity of the very files the timed steps wrote: md5 against the unmodified reference's output for this workload (committed; made on the CPU box)
     parity = {"checked": False}
@@ -402,7 +439,10 @@ def main():
             "candidates": int(results[-1]["n_cand"]), "unfiltered_candidates": int(st.n_unfiltered_candidates), "fragments_per_step": n_frag, "wall_seconds_timed_region": wall}
     if secondary:
         line["secondary_mode"] = secondary
-    if not args.no_cpu_baseline and world == 1:   # the CPU reference beside the GPU number: rank 0 at N=1 only
+    if not args.no_cpu_baseline and world == 1 and not _build.oracle_available():
+        line["cpu_baseline"] = {"value": None, "unit": UNIT, "cores": 1, "kind": "reference", "sample": None,
+                                "not_measured": "the reference binary oracle/_ref/arriba is not built here (oracle/Makefile needs the reference sources)", "full_size": REFERENCE_FULL_SIZE.get(args.workload)}
+    elif not args.no_cpu_baseline and world == 1:   # the CPU reference beside the GPU number: rank 0 at N=1 only
         sp = ensure_world(args.workload, sample_bp)
         n, scope_s, total = reference_run(sp, cores)
         line["cpu_baseline"] = {"value": n / scope_s, "unit": UNIT, "cores": 1, "kind": "reference",

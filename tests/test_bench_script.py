@@ -2,6 +2,8 @@
 leg with the reference binary, the JSON line as the last line of stdout, a quiet stderr) on the CPU stand-in: tests/bench_dry_run.py swaps the library and
 pretends a device is there. The numbers mean nothing; a typo in the script would otherwise only show on the GPU box at the end of a round."""
 import json, os, subprocess, sys
+import pytest
+from arriba_b200 import _build
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -21,6 +23,26 @@ def test_bench_script_runs_on_the_stand_in(hostsim_lib, tmp_path):
     assert {"bound", "achieved", "peak", "unit", "frac", "traffic"} <= set(line["roofline"]) and {"value", "unit", "cores", "kind", "sample"} <= set(line["cpu_baseline"])
 
 
+def test_bench_dump_outputs(hostsim_lib, tmp_path):
+    """--dump-outputs: the last timed step's candidate table and labels as float64 .npy files, the same for two runs with the same arguments"""
+    import numpy as np
+    env = dict(os.environ, ARB_BENCH_DIR=str(tmp_path), PYTHONPATH=ROOT)
+    dumps = []
+    for run, steps in (("a", "1"), ("b", "2")):
+        d = str(tmp_path / run)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "bench_dry_run.py"), "--workload", "tiny_20k", "--steps", steps, "--warmup", "0", "--no-cpu-baseline",
+                            "--dump-outputs", d], env=env, capture_output=True, text=True, timeout=900, cwd=str(tmp_path))
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == int(steps)
+        dumps.append({f: np.load(os.path.join(d, f)) for f in sorted(os.listdir(d))})
+    assert sorted(dumps[0]) == sorted(dumps[1]) and "candidates.filter.npy" in dumps[0] and "fragments.label.npy" in dumps[0]
+    assert sum(a.nbytes for a in dumps[0].values()) <= 64 << 20
+    for f, a in dumps[0].items():
+        assert a.dtype == np.float64 and np.array_equal(a, dumps[1][f]), f
+    assert len(dumps[0]["fragments.label.npy"]) > 10000
+
+
+@pytest.mark.skipif(not _build.oracle_available(), reason="needs the reference binary, which oracle/Makefile builds from the reference sources")
 def test_reference_arm_line(tmp_path):
     env = dict(os.environ, ARB_BENCH_DIR=str(tmp_path), PYTHONPATH=ROOT)
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "tiny_20k", "--steps", "1", "--warmup", "0"], env=env, capture_output=True, text=True, timeout=900, cwd=str(tmp_path))

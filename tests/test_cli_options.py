@@ -36,14 +36,13 @@ def test_cli_option_parity(worlds, cli, tmp_path, extra):
     out = str(tmp_path / "fusions.tsv"); disc = str(tmp_path / "fusions.discarded.tsv")
     r = subprocess.run([cli, "-x", w.prefix + ".bam", "-g", w.prefix + ".gtf", "-a", w.prefix + ".fa", "-o", out, "-O", disc, "-@", "3"] + list(args), capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
-    assert open(out, "rb").read() == open(os.path.join(w.outdir, "fusions.tsv"), "rb").read(), "fusions.tsv differs with options %s" % (args,)
-    assert open(disc, "rb").read() == open(os.path.join(w.outdir, "fusions.discarded.tsv"), "rb").read(), "fusions.discarded.tsv differs with options %s" % (args,)
+    assert w.same_output("fusions.tsv", out), "fusions.tsv differs with options %s" % (args,)
+    assert w.same_output("fusions.discarded.tsv", disc), "fusions.discarded.tsv differs with options %s" % (args,)
 
 
 def test_cli_error_parity(worlds, cli, tmp_path):
     """Unusable inputs: same ERROR line and exit code as the reference (common.hpp:330, read_chimeric_alignments.cpp:566-609, annotation.cpp, assembly.cpp)."""
     w = worlds.get("small")
-    oracle = _build.build_oracle()
     d = str(tmp_path)
     bam = open(w.prefix + ".bam", "rb").read()
     gtf = open(w.prefix + ".gtf").read().split("\n")
@@ -67,10 +66,10 @@ def test_cli_error_parity(worlds, cli, tmp_path):
              (d + "/truncated.bam", w.prefix + ".gtf", w.prefix + ".fa"), (d + "/empty.bam", w.prefix + ".gtf", w.prefix + ".fa"), (d + "/garbage.bam", w.prefix + ".gtf", w.prefix + ".fa"),
              (w.prefix + ".bam", d + "/empty.gtf", w.prefix + ".fa"), (w.prefix + ".bam", d + "/no_exons.gtf", w.prefix + ".fa"), (w.prefix + ".bam", w.prefix + ".gtf", d + "/two_contigs.fa")]
     for b, g, a in cases:
-        seen = []
-        for exe in (oracle, cli):
-            r = subprocess.run([exe, "-x", b, "-g", g, "-a", a, "-o", d + "/o.tsv", "-O", d + "/d.tsv", "-f", "blacklist"] + (["-@", "2"] if exe == cli else []), capture_output=True, text=True, timeout=300)
-            seen.append((r.returncode, [l for l in r.stderr.split("\n") if l.startswith("ERROR")]))
+        rc, errors, _ = worldutil.reference_cli(b, g, a, ["-f", "blacklist"])
+        seen = [(rc, errors)]
+        r = subprocess.run([cli, "-x", b, "-g", g, "-a", a, "-o", d + "/o.tsv", "-O", d + "/d.tsv", "-f", "blacklist", "-@", "2"], capture_output=True, text=True, timeout=300)
+        seen.append((r.returncode, [l for l in r.stderr.split("\n") if l.startswith("ERROR")]))
         assert seen[0] == seen[1], (b, g, a, seen)
         assert seen[0][0] == 1 or b.endswith("only_chimeric.bam"), (b, g, a, seen)   # chimeric mates count as mapped reads: the reference runs through (and so must the product)
 
@@ -96,17 +95,17 @@ def random_options(rng):
 def run_random_combination(rng, cli, d, k):
     """one random world, one random option set, reference and product side by side; True when both stop with the same error or both write the same two files"""
     from test_random_worlds import random_world_arguments
-    oracle = _build.build_oracle()
     kw = random_world_arguments(rng); pre = os.path.join(d, "w%d" % k)
     worldutil.run_synth(pre, **{kk: v for kk, v in kw.items() if kk != "extra"}, extra=kw["extra"])
-    opts = random_options(rng); res = []
-    for exe, tag in ((oracle, "r"), (cli, "p")):
-        r = subprocess.run([exe, "-x", pre + ".bam", "-g", pre + ".gtf", "-a", pre + ".fa", "-o", pre + "." + tag + ".tsv", "-O", pre + "." + tag + ".d.tsv"] + opts + (["-@", str(rng.choice([1, 3, 6]))] if exe == cli else []),
-                           capture_output=True, text=True, env=dict(os.environ, ARB_DET_ALLOC="1"), timeout=900)
-        res.append((r.returncode, [l for l in r.stderr.splitlines() if l.startswith("ERROR")]))
+    opts = random_options(rng)
+    rc, errors, sha = worldutil.reference_cli(pre + ".bam", pre + ".gtf", pre + ".fa", opts, det_alloc=True)
+    res = [(rc, errors)]
+    r = subprocess.run([cli, "-x", pre + ".bam", "-g", pre + ".gtf", "-a", pre + ".fa", "-o", pre + ".p.tsv", "-O", pre + ".p.d.tsv"] + opts + ["-@", str(rng.choice([1, 3, 6]))],
+                       capture_output=True, text=True, env=dict(os.environ, ARB_DET_ALLOC="1"), timeout=900)
+    res.append((r.returncode, [l for l in r.stderr.splitlines() if l.startswith("ERROR")]))
     if res[0][0] != 0 or res[1][0] != 0:
         return res[0] == res[1], opts, kw
-    same = all(open(pre + ".r" + e, "rb").read() == open(pre + ".p" + e, "rb").read() for e in (".tsv", ".d.tsv"))
+    same = sha == {"fusions.tsv": worldutil.file_digest(pre + ".p.tsv"), "fusions.discarded.tsv": worldutil.file_digest(pre + ".p.d.tsv")}
     return same, opts, kw
 
 

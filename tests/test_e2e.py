@@ -10,16 +10,9 @@ def check_e2e(world, lib_path, tmp_path, threads=4):
     p = L.Pipeline(world.prefix + ".bam", world.prefix + ".gtf", world.prefix + ".fa", threads=threads, lib_path=lib_path, output=out, discarded=disc)
     p.run_all()
     p.close()
-    want = open(os.path.join(world.outdir, "fusions.tsv")).read().split("\n")
-    got = open(out).read().split("\n")
-    assert len(want) > 5
-    for i, (g, w) in enumerate(zip(got, want)):
-        if g != w:
-            gc, wc = g.split("\t"), w.split("\t")
-            cols = [j for j in range(min(len(gc), len(wc))) if gc[j] != wc[j]]
-            raise AssertionError("fusions.tsv line %d differs in columns %s:\n got  %s\n want %s" % (i + 1, cols, [gc[j][:200] for j in cols], [wc[j][:200] for j in cols]))
-    assert len(got) == len(want)
-    assert open(disc).read() == open(os.path.join(world.outdir, "fusions.discarded.tsv")).read(), "discarded file differs"
+    assert world.output_lines("fusions.tsv") > 5
+    assert world.same_output("fusions.tsv", out), "fusions.tsv differs from the reference's"
+    assert world.same_output("fusions.discarded.tsv", disc), "discarded file differs"
 
 
 def test_e2e_hostsim(worlds, hostsim_lib, tmp_path):
@@ -94,8 +87,8 @@ def test_cli_cuda(worlds, tmp_path, extra):
     r = subprocess.run([_build.build_cli(), "-x", w.prefix + ".bam", "-g", w.prefix + ".gtf", "-a", w.prefix + ".fa", "-o", out, "-O", disc, "-@", "4"] + list(args),
                        capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
-    assert open(out, "rb").read() == open(os.path.join(w.outdir, "fusions.tsv"), "rb").read()
-    assert open(disc, "rb").read() == open(os.path.join(w.outdir, "fusions.discarded.tsv"), "rb").read()
+    assert w.same_output("fusions.tsv", out)
+    assert w.same_output("fusions.discarded.tsv", disc)
 
 
 def test_e2e_hostsim_compressed_chr_names_normal_pairs(worlds, hostsim_lib, tmp_path):

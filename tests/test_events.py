@@ -1,26 +1,34 @@
 """Event-level chain: after every stage the candidate table (filter, read counts, e-value) must equal the oracle's."""
 import numpy as np
 import pytest
-import worldutil
 from arriba_b200 import lib as L
-from test_find_fusions import key_of
+from test_find_fusions import KEY, by_key
+from worldutil import digest
+
+COLUMNS = ("filter", "split_reads1", "split_reads2", "discordant_mates")
+
+
+def stage_digests(t, with_evalue, with_confidence):
+    """a candidate table in key order: keys, filter, read counts, supporting list sizes (and e-values, confidence)"""
+    o = by_key(t)
+    out = {c: digest(np.asarray(t[c])[o]) for c in KEY + COLUMNS + (("evalue",) if with_evalue else ()) + (("confidence",) if with_confidence else ())}
+    for oname in ("list1_off", "list2_off"):
+        out[oname + " sizes"] = digest(np.diff(np.asarray(t[oname]).astype(np.int64))[o])
+    return out
+
+
+def reference_stage(name, occ, with_evalue):
+    def compute(w):
+        t = w.stage("ev_" + name, occ)
+        return {"candidates": stage_digests(t, with_evalue, name == "confidence"), "remaining": int(t["remaining"][0]),
+                "frag_filter": digest(t["frag_filter"]) if "frag_filter" in t else None}
+    return compute
 
 
 def compare_stage(got, want, stage, check_evalue):
-    index = {key_of(want, i): i for i in range(len(want["gene1"]))}
-    perm = np.array([index[key_of(got, i)] for i in range(got["n"])])
-    for name in ("filter", "split_reads1", "split_reads2", "discordant_mates"):
-        w = want[name][perm]
-        bad = np.nonzero(got[name] != w)[0]
-        assert len(bad) == 0, (stage, name, len(bad), [key_of(got, i) for i in bad[:5]], got[name][bad[:5]], w[bad[:5]])
-    if check_evalue:
-        w = want["evalue"][perm]
-        bad = np.nonzero(got["evalue"].view(np.uint32) != w.view(np.uint32))[0]
-        assert len(bad) == 0, (stage, "evalue", len(bad), got["evalue"][bad[:5]], w[bad[:5]], [key_of(got, i) for i in bad[:5]])
-    for lname, oname in (("list1", "list1_off"), ("list2", "list2_off")):
-        gs = np.diff(got[oname].astype(np.int64)); ws = np.diff(want[oname].astype(np.int64))[perm]
-        assert np.array_equal(gs, ws), (stage, lname + " sizes")
-    return perm
+    mine = stage_digests(got, check_evalue, stage == "confidence")
+    bad = [k for k in want if mine[k] != want[k]]
+    assert not bad, (stage, "candidate columns differ from the reference's", bad)
 
 
 def check_events(world, lib_path, threads=4, keep=False):
@@ -28,10 +36,9 @@ def check_events(world, lib_path, threads=4, keep=False):
     p.run(L.STEP_FIND_FUSIONS)
     p.events(0)
     got = p.candidates()
-    ff = world.stage("find_fusions")
     # the replayed unordered_map iteration order must be the reference's
-    want_keys = [key_of(ff, i) for i in range(len(ff["gene1"]))]
-    got_keys = [key_of(got, int(i)) for i in got["order"]]
+    want_keys = world.fact("find_fusions/order", lambda w: {k: digest(w.stage("find_fusions")[k]) for k in KEY})
+    got_keys = {k: digest(got[k][got["order"]]) for k in KEY}
     assert got_keys == want_keys, "iteration order of the candidate table differs from the reference's unordered_map"
     stages = ["merge_adjacent", "multimappers", "evalue", "non_coding_neighbors", "intragenic_exonic", "min_support", "relative_support", "internal_tandem_duplication",
               "intronic", "in_vitro", "spliced", "select_best", "marginal_read_through", "many_spliced", "short_anchor", "end_to_end", "no_coverage",
@@ -44,14 +51,12 @@ def check_events(world, lib_path, threads=4, keep=False):
         if name == "kmer_index":
             continue
         occ = occurrence.get(name, 0); occurrence[name] = occ + 1
-        want = world.stage("ev_" + name, occ)
         seen_evalue = seen_evalue or name == "evalue"
-        compare_stage(got, want, name, seen_evalue)
-        if "frag_filter" in want:
-            assert np.array_equal(got["labels"], want["frag_filter"]), (name, "fragment labels")
-        assert int((got["filter"] == 0).sum()) == int(want["remaining"][0]) or name in ("evalue", "confidence"), name
-        if name == "confidence":
-            assert np.array_equal(got["confidence"], want["confidence"][compare_stage(got, want, name, True)])
+        want = world.fact("ev_%s/%d/candidates" % (name, occ), reference_stage(name, occ, seen_evalue))
+        compare_stage(got, want["candidates"], name, seen_evalue)
+        if want["frag_filter"] is not None:
+            assert digest(got["labels"]) == want["frag_filter"], (name, "fragment labels")
+        assert int((got["filter"] == 0).sum()) == want["remaining"] or name in ("evalue", "confidence"), name
     if keep:
         return p
     p.close()
@@ -71,9 +76,10 @@ CFG5 = dict(scale=0.002, genes=800, breakpoints=400, fragments=40000, extra=("--
 def test_events_hostsim_mismapper_heavy(worlds, hostsim_lib):
     """BASELINE.json configs[4] in miniature: homologous partners, clipped segments alignable in the donor, adjacent breakpoints, ITD merges."""
     w = worlds.get("cfg5", **CFG5)
-    mm = w.stage("ev_mismappers")
-    assert (mm["frag_filter"] == 11).sum() > 1000 and (mm["filter"] == 11).sum() > 20 and (w.stage("ev_homologs")["filter"] == 37).sum() > 5
-    assert (w.stage("ev_merge_adjacent")["filter"] == 23).sum() > 20
+    n = w.fact("ev/mismapper_heavy_counts", lambda w: [int((w.stage("ev_mismappers")["frag_filter"] == 11).sum()), int((w.stage("ev_mismappers")["filter"] == 11).sum()),
+                                                       int((w.stage("ev_homologs")["filter"] == 37).sum()), int((w.stage("ev_merge_adjacent")["filter"] == 23).sum())])
+    assert n[0] > 1000 and n[1] > 20 and n[2] > 5
+    assert n[3] > 20
     check_events(w, hostsim_lib)
 
 

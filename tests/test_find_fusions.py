@@ -2,6 +2,7 @@
 import numpy as np
 import pytest
 import worldutil
+from worldutil import digest
 
 
 def key_of(t, i):
@@ -9,49 +10,69 @@ def key_of(t, i):
             int(t["direction1"][i]), int(t["direction2"][i]))
 
 
+KEY = ("gene1", "gene2", "contig1", "contig2", "breakpoint1", "breakpoint2", "direction1", "direction2")
+
+
+def by_key(t):
+    """permutation that sorts a candidate table by its 8-tuple key"""
+    return np.lexsort([np.asarray(t[k]).astype(np.int64) for k in reversed(KEY)])
+
+
+def candidate_digests(t, bits, bits2):
+    """digests of a candidate table in key order: keys, read counts, filter, anchors, exonic / spliced / strand bits and the supporting lists"""
+    o = by_key(t)
+    out = {k: digest(np.asarray(t[k])[o]) for k in KEY + ("split_reads1", "split_reads2", "discordant_mates", "filter", "anchor_start1", "anchor_start2")}
+    out["bits"] = digest(np.asarray(bits)[o]); out["bits2"] = digest(np.asarray(bits2)[o])
+    for lname, oname in (("list1", "list1_off"), ("list2", "list2_off"), ("listd", "listd_off")):
+        off = np.asarray(t[oname]).astype(np.int64)
+        out[lname] = digest(worldutil._segments(t[lname], off[:-1][o], np.diff(off)[o]))
+        out[lname + "_sizes"] = digest(np.diff(off)[o])
+    out["n"] = len(o); out["n_unique"] = len(set(zip(*[np.asarray(t[k]).tolist() for k in KEY])))
+    return out
+
+
+def reference_candidates(w):
+    ff = w.stage("find_fusions")
+    bits = (ff["exonic1"].astype(np.int64) | ff["exonic2"].astype(np.int64) << 1 | ff["spliced1"].astype(np.int64) << 2 | ff["spliced2"].astype(np.int64) << 3 |
+            ff["predicted_strand1"].astype(np.int64) << 4 | ff["predicted_strand2"].astype(np.int64) << 5 | ff["predicted_strands_ambiguous"].astype(np.int64) << 6 |
+            ff["transcript_start"].astype(np.int64) << 7)
+    return candidate_digests(ff, bits, ff["transcript_start_ambiguous"])
+
+
+def reference_swaps(w):
+    """mate canonicalisation in the reference (fusions.cpp:416-421): the fragments whose first alignment changed"""
+    ff, ann = w.stage("find_fusions"), w.stage("annotated")
+    first = ann["aln_off"][:-1]
+    swapped = (ff["slot0_start"] != ann["start"][first]) | (ff["slot0_contig"] != ann["contig"][first])
+    return {"swapped": digest(np.nonzero(swapped)[0]), "n": int(swapped.sum())}
+
+
 def check_find_fusions(world, lib_path):
-    ctx = worldutil.context_from_oracle(world, lib_path)
-    # start from the oracle's labels so that this test isolates find_fusions
-    ctx.set_fragment_filters(world.stage("rf_low_entropy")["frag_filter"])
-    ff = world.stage("find_fusions")
-    ctx.find_fusions(int(ff["max_mate_gap"][0]))
+    p = worldutil.front_end(world, lib_path)
+    fr = p.fragments(); n = fr["n_fragments"]
+    # a swap of two mates with identical start and contig is not observable in the reference's dump
+    twins = (fr["start"][:n] == fr["start"][n:2 * n]) & (fr["contig"][:n] == fr["contig"][n:2 * n]) & (fr["n_aln"] > 1)
+    ctx = p.context()
+    # start from the reference's labels so that this test isolates find_fusions
+    ctx.run_read_filters()
+    labels, _ = ctx.fragment_filters()
+    assert digest(labels) == world.stage_digest("rf_low_entropy", "frag_filter")
+    ctx.set_fragment_filters(labels)
+    ctx.find_fusions(world.stage_scalar("find_fusions", "max_mate_gap"))
     got = ctx.candidates()
-    assert got["n"] == len(ff["gene1"])
-    want_index = {key_of(ff, i): i for i in range(len(ff["gene1"]))}
-    assert len(want_index) == len(ff["gene1"])
-    n_checked_lists = 0
-    for i in range(got["n"]):
-        j = want_index[key_of(got, i)]
-        ctxmsg = "candidate %s" % (key_of(got, i),)
-        for name in ("split_reads1", "split_reads2", "discordant_mates", "filter"):
-            assert int(got[name][i]) == int(ff[name][j]), (ctxmsg, name, int(got[name][i]), int(ff[name][j]))
-        assert int(got["anchor_start1"][i]) == int(ff["anchor_start1"][j]) and int(got["anchor_start2"][i]) == int(ff["anchor_start2"][j]), ctxmsg
-        b = int(got["bits"][i])
-        want_bits = (int(ff["exonic1"][j]) | int(ff["exonic2"][j]) << 1 | int(ff["spliced1"][j]) << 2 | int(ff["spliced2"][j]) << 3 |
-                     int(ff["predicted_strand1"][j]) << 4 | int(ff["predicted_strand2"][j]) << 5 | int(ff["predicted_strands_ambiguous"][j]) << 6 |
-                     int(ff["transcript_start"][j]) << 7)
-        assert b == want_bits, (ctxmsg, bin(b), bin(want_bits))
-        assert int(got["bits2"][i]) == int(ff["transcript_start_ambiguous"][j]), ctxmsg
-        for lname, oname in (("list1", "list1_off"), ("list2", "list2_off"), ("listd", "listd_off")):
-            g = got[lname][got[oname][i]:got[oname][i + 1]]
-            w = ff[lname][ff[oname][j]:ff[oname][j + 1]]
-            assert np.array_equal(g, w), (ctxmsg, lname, g[:10], w[:10])
-            n_checked_lists += len(w)
-    assert n_checked_lists > 0
+    want = world.fact("find_fusions/candidates", reference_candidates)
+    assert want["n_unique"] == want["n"] and got["n"] == want["n"]
+    mine = candidate_digests(got, got["bits"], got["bits2"])
+    bad = [k for k in want if mine[k] != want[k]]
+    assert not bad, ("candidate columns differ from the reference's", bad)
+    assert want["n"] > 0
     # candidates are numbered in the reference's first-insertion order: first supporting fragment ascending
     # mate canonicalisation (fusions.cpp:416-421)
-    ann = world.stage("annotated")
-    slot0_before = ann["start"][ann["aln_off"][:-1]]
-    swapped_want = (ff["slot0_start"] != slot0_before) | (ff["slot0_contig"] != ann["contig"][ann["aln_off"][:-1]])
+    ref = world.fact("find_fusions/swaps", reference_swaps)
     swapped_got = ctx.slot_swaps().astype(bool)
-    # a swap of two mates with identical start and contig is not observable in the dump
-    assert np.all(swapped_got[swapped_want]), "missing canonicalisation"
-    extra = np.nonzero(swapped_got & ~swapped_want)[0]
-    for i in extra:
-        a = ann["aln_off"][i]
-        assert ann["start"][a] == ann["start"][a + 1] and ann["contig"][a] == ann["contig"][a + 1]
-    assert int((got["filter"] == 0).sum()) == int(ff["remaining"][0])
-    ctx.close()
+    assert digest(np.nonzero(swapped_got & ~twins)[0]) == ref["swapped"], "canonicalisation differs from the reference's"
+    assert int((got["filter"] == 0).sum()) == world.stage_scalar("find_fusions", "remaining")
+    p.close()
 
 
 def test_find_fusions_hostsim(worlds, hostsim_lib):

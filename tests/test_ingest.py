@@ -3,54 +3,11 @@ and of the whole file-to-candidates path."""
 import numpy as np
 import pytest
 import worldutil
+from worldutil import digest
 from arriba_b200 import lib as L
 
 
-def frag_tables_equal(got, d, check_genes, check_pred):
-    """got: Pipeline.fragments(); d: oracle fragment dump."""
-    n = len(d["n_aln"])
-    assert got["n_fragments"] == n, (got["n_fragments"], n)
-    names_want = bytes(d["names"])
-    assert got["names_blob"] == names_want, "fragment names / name order differ"
-    assert np.array_equal(got["name_off"], d["name_off"].astype(np.uint64))
-    want = worldutil.chunk_from_dump(d)
-    assert np.array_equal(got["n_aln"], want["n_aln"])
-    assert np.array_equal(got["fflags"], want["fflags"]), np.nonzero(got["fflags"] != want["fflags"])[0][:10]
-    valid = np.zeros(3 * n, bool)
-    for s in range(3):
-        valid[s * n:(s + 1) * n] = want["n_aln"] > s
-    for k in ("contig", "start", "end", "cigar_cnt"):
-        bad = np.nonzero((got[k] != want[k]) & valid)[0]
-        assert len(bad) == 0, (k, bad[:10] % n, bad[:10] // n, got[k][bad[:10]], want[k][bad[:10]])
-    mask = 0b001011 | (0b000100 if check_genes else 0) | (0b100000 if check_pred else 0)
-    ga, wa = got["aflags"] & mask, want["aflags"] & mask
-    bad = np.nonzero((ga != wa) & valid)[0]
-    assert len(bad) == 0, ("aflags", bad[:10] % n, bad[:10] // n, got["aflags"][bad[:10]], want["aflags"][bad[:10]])
-    if check_pred:  # predicted strand only meaningful when not ambiguous
-        unamb = valid & ((want["aflags"] & 32) == 0)
-        bad = np.nonzero(((got["aflags"] ^ want["aflags"]) & 16 != 0) & unamb)[0]
-        assert len(bad) == 0, ("predicted strand", bad[:10] % n, bad[:10] // n)
-    # CIGARs and sequences, alignment by alignment
-    for x in np.nonzero(valid)[0]:
-        a = got["cigar"][got["cigar_off"][x]:got["cigar_off"][x] + got["cigar_cnt"][x]]
-        b = want["cigar"][want["cigar_off"][x]:want["cigar_off"][x] + want["cigar_cnt"][x]]
-        if not np.array_equal(a, b):
-            raise AssertionError(("cigar", x % n, x // n, a, b))
-    v2 = valid[:2 * n]
-    assert np.array_equal(got["seq_len"][v2], want["seq_len"][v2])
-    for x in np.nonzero(v2)[0][:20000]:
-        nb = (int(want["seq_len"][x]) + 1) // 2
-        a = got["seq"][int(got["seq_off"][x]) * 16:int(got["seq_off"][x]) * 16 + nb]
-        b = want["seq"][int(want["seq_off"][x]) * 16:int(want["seq_off"][x]) * 16 + nb]
-        if not np.array_equal(a, b):
-            raise AssertionError(("seq", x % n, x // n))
-    if check_genes:
-        assert np.array_equal(got["genes_cnt"][valid], want["genes_cnt"][valid]), "gene set sizes differ"
-        for x in np.nonzero(valid)[0]:
-            a = got["genes"][got["genes_off"][x]:got["genes_off"][x] + got["genes_cnt"][x]]
-            b = want["genes"][want["genes_off"][x]:want["genes_off"][x] + want["genes_cnt"][x]]
-            if not np.array_equal(a, b):
-                raise AssertionError(("genes", x % n, x // n, a, b))
+frag_tables_equal = worldutil.frag_tables_equal
 
 
 def check_front_end(world, lib_path, threads):
@@ -58,47 +15,48 @@ def check_front_end(world, lib_path, threads):
     p.step(L.STEP_LOAD_REFERENCE)
     p.step(L.STEP_INGEST)
     st = p.stats()
-    rca = world.stage("read_chimeric_alignments")
-    assert st.mapped_reads == int(rca["mapped_reads"][0])
-    assert st.n_fragments == int(rca["total"][0])
-    frag_tables_equal(p.fragments(), world.stage("ingest"), check_genes=False, check_pred=False)
-    # coverage windows
-    off = rca["coverage_off"]
-    for c in range(len(off) - 1):
-        cov, starts, ends = p.coverage(c)
-        want = rca["coverage"][off[c]:off[c + 1]]
-        assert len(cov) == len(want), (c, len(cov), len(want))
-        assert np.array_equal(cov, want), ("coverage", c, np.nonzero(cov != want)[0][:10])
-        assert np.array_equal(starts, rca["fragment_starts"][off[c]:off[c + 1]]), ("starts", c)
-        assert np.array_equal(ends, rca["fragment_ends"][off[c]:off[c + 1]]), ("ends", c)
+    assert st.mapped_reads == world.stage_scalar("read_chimeric_alignments", "mapped_reads")
+    assert st.n_fragments == world.stage_scalar("read_chimeric_alignments", "total")
+    frag_tables_equal(p.fragments(), world, "ingest", check_genes=False, check_pred=False)
+    # coverage windows, contig by contig
+    def coverage_ref(w):
+        rca = w.stage("read_chimeric_alignments")
+        return {"sizes": digest(np.diff(rca["coverage_off"].astype(np.int64))), "coverage": digest(rca["coverage"]),
+                "starts": digest(rca["fragment_starts"]), "ends": digest(rca["fragment_ends"]), "n_contigs": len(rca["coverage_off"]) - 1}
+    want = world.fact("coverage", coverage_ref)
+    windows = [p.coverage(c) for c in range(want["n_contigs"])]
+    got = {"sizes": digest([len(w[0]) for w in windows]), "n_contigs": want["n_contigs"]}
+    for i, k in enumerate(("coverage", "starts", "ends")):
+        got[k] = digest(np.concatenate([w[i] for w in windows]) if windows else [])
+    assert got == want, [k for k in want if got[k] != want[k]]
     p.step(L.STEP_ANNOTATE)
-    assert p.stats().strandedness == int(world.stage("strandedness")["strandedness"][0])
-    frag_tables_equal(p.fragments(), world.stage("annotated"), check_genes=True, check_pred=True)
-    fl = world.stage("fragment_length")
+    assert p.stats().strandedness == world.stage_scalar("strandedness", "strandedness")
+    frag_tables_equal(p.fragments(), world, "annotated", check_genes=True, check_pred=True)
     g = p.genes()
-    assert g["n_genes"] == len(fl["gene_id"])
-    for k, w in (("gene_contig", "gene_contig"), ("gene_start", "gene_start"), ("gene_end", "gene_end"), ("gene_strand", "gene_strand"), ("gene_exonic_length", "gene_exonic_length")):
-        assert np.array_equal(g[k], fl[w]), k
-    assert np.array_equal(g["gene_flags"], fl["gene_is_dummy"] | fl["gene_is_protein_coding"] << 1)
-    want_ann = worldutil.annotation_from_dump(fl, g["n_contigs"])
-    for k in ("exon_gene", "exon_start", "exon_end", "exon_cds_start", "exon_cds_end", "exon_flags"):
-        assert np.array_equal(g[k], want_ann[k]), k
+    assert g["n_genes"] == world.fact("fragment_length/n_genes", lambda w: len(w.stage("fragment_length")["gene_id"]))
+    for k in ("gene_contig", "gene_start", "gene_end", "gene_strand", "gene_exonic_length"):
+        assert digest(g[k]) == world.stage_digest("fragment_length", k), k
+    assert digest(g["gene_flags"]) == world.fact("fragment_length/gene_flags", lambda w: digest(w.stage("fragment_length")["gene_is_dummy"] | w.stage("fragment_length")["gene_is_protein_coding"] << 1))
+    exon_columns = ("exon_gene", "exon_start", "exon_end", "exon_cds_start", "exon_cds_end", "exon_flags")
+    want_ann = world.fact("fragment_length/exons", lambda w: {k: digest(v) for k, v in worldutil.annotation_from_dump(w.stage("fragment_length"), g["n_contigs"]).items() if k in exon_columns})
+    for k in exon_columns:
+        assert digest(g[k]) == want_ann[k], k
     # device stages fed by the product's own front end
     p.step(L.STEP_UPLOAD); p.step(L.STEP_READ_FILTERS); p.step(L.STEP_FRAGMENT_LENGTH)
     ctx = p.context()
     labels, early = ctx.fragment_filters()
-    assert np.array_equal(labels, world.stage("rf_low_entropy")["frag_filter"])
+    assert digest(labels) == world.stage_digest("rf_low_entropy", "frag_filter")
     st = p.stats()
-    assert st.fragment_length_ok == int(fl["ok"][0])
+    assert st.fragment_length_ok == world.stage_scalar("fragment_length", "ok")
     if st.fragment_length_ok:
-        assert st.mate_gap_mean == fl["gap_mean_stddev_readlen"][0] and st.mate_gap_stddev == fl["gap_mean_stddev_readlen"][1]
-        assert st.read_length_mean == fl["gap_mean_stddev_readlen"][2]
-    ff = world.stage("find_fusions")
-    assert st.max_mate_gap == int(ff["max_mate_gap"][0])
+        gap = world.fact("fragment_length/gap_mean_stddev_readlen", lambda w: [float(x) for x in w.stage("fragment_length")["gap_mean_stddev_readlen"]])
+        assert st.mate_gap_mean == gap[0] and st.mate_gap_stddev == gap[1]
+        assert st.read_length_mean == gap[2]
+    assert st.max_mate_gap == world.stage_scalar("find_fusions", "max_mate_gap")
     p.step(L.STEP_FIND_FUSIONS)
     cand = ctx.candidates()
-    assert cand["n"] == len(ff["gene1"])
-    assert int((cand["filter"] == 0).sum()) == int(ff["remaining"][0])
+    assert cand["n"] == world.fact("find_fusions/n", lambda w: len(w.stage("find_fusions")["gene1"]))
+    assert int((cand["filter"] == 0).sum()) == world.stage_scalar("find_fusions", "remaining")
     p.close()
 
 

@@ -28,7 +28,7 @@ def run_one(cache, name, kw, lib_path, threads, outdir):
     out = os.path.join(outdir, "fusions.tsv"); disc = os.path.join(outdir, "fusions.discarded.tsv")
     p = L.Pipeline(w.prefix + ".bam", w.prefix + ".gtf", w.prefix + ".fa", threads=threads, lib_path=lib_path, output=out, discarded=disc)
     p.run_all(); p.close()
-    return open(out, "rb").read() == open(os.path.join(w.outdir, "fusions.tsv"), "rb").read() and open(disc, "rb").read() == open(os.path.join(w.outdir, "fusions.discarded.tsv"), "rb").read()
+    return w.same_output("fusions.tsv", out) and w.same_output("fusions.discarded.tsv", disc)
 
 
 @pytest.mark.parametrize("seed", [11, 12, 13, 14])

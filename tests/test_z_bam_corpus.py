@@ -23,8 +23,7 @@ def transcoded_world(worlds, tmp_root, seed, eof=True, **kw):
     if not os.path.exists(prefix + ".bam"):
         n = bamtools.transcode(base.prefix + ".bam", prefix + ".bam", seed, eof)
         assert n > 1000
-        worldutil.run_oracle(prefix, os.path.join(d, "oracle"))
-    return base, worldutil.World(prefix, os.path.join(d, "oracle"))
+    return base, worldutil.reference_world(prefix, os.path.join(d, "oracle"))
 
 
 @pytest.fixture(scope="module")
@@ -48,8 +47,8 @@ def test_python_reader_round_trip(worlds, tmp_path):
 def test_oracle_reads_the_transcoded_file_the_same(corpus, which):
     base, tr = corpus[which]
     for name in ("fusions.tsv", "fusions.discarded.tsv"):
-        assert open(os.path.join(tr.outdir, name), "rb").read() == open(os.path.join(base.outdir, name), "rb").read(), name
-    assert len(open(os.path.join(tr.outdir, "fusions.tsv")).read().split("\n")) > 5
+        assert tr.output_digest(name) == base.output_digest(name), name
+    assert tr.output_lines("fusions.tsv") > 5
 
 
 @pytest.mark.parametrize("which,threads", [((1, True), 3), ((2, False), 1)])
@@ -86,9 +85,8 @@ def mutated_world(worlds, root, mutation_seed, rate, **kw):
         os.symlink(base.prefix + ext, prefix + ext)
     tally = bamtools.mutate(base.prefix + ".bam", prefix + ".bam", mutation_seed, rate)
     assert set(tally) == set(bamtools.MUTATIONS) and min(tally.values()) > 50, tally
-    worldutil.run_oracle(prefix, os.path.join(d, "oracle"))
-    w = worldutil.World(prefix, os.path.join(d, "oracle"))
-    assert "SAM records were malformed" in open(os.path.join(w.outdir, "stderr.txt")).read()   # the repair / rejection rules did fire in the reference
+    w = worldutil.reference_world(prefix, os.path.join(d, "oracle"))
+    assert w.stderr_has("SAM records were malformed")   # the repair / rejection rules did fire in the reference
     return w
 
 

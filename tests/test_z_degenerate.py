@@ -18,8 +18,8 @@ def check(world, lib_path, tmp_path, threads):
     out = os.path.join(str(tmp_path), "fusions.tsv"); disc = os.path.join(str(tmp_path), "fusions.discarded.tsv")
     p = L.Pipeline(world.prefix + ".bam", world.prefix + ".gtf", world.prefix + ".fa", threads=threads, lib_path=lib_path, output=out, discarded=disc)
     p.run_all(); p.close()
-    assert open(out, "rb").read() == open(os.path.join(world.outdir, "fusions.tsv"), "rb").read()
-    assert open(disc, "rb").read() == open(os.path.join(world.outdir, "fusions.discarded.tsv"), "rb").read()
+    assert world.same_output("fusions.tsv", out)
+    assert world.same_output("fusions.discarded.tsv", disc)
     return len(open(out).read().splitlines()) - 1
 
 

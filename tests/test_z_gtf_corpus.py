@@ -23,11 +23,9 @@ def damaged(worlds, tmp_path_factory):
             os.symlink(base.prefix + ".fa", prefix + ".fa")
         tally = gtftools.damage_gtf(base.prefix + ".gtf", prefix + ".gtf", seed, rate, lengths)
         assert set(tally) == set(gtftools.KINDS), tally
-        worldutil.run_oracle(prefix, os.path.join(d, "oracle"))
-        out[seed] = worldutil.World(prefix, os.path.join(d, "oracle"))
-        err = open(os.path.join(out[seed].outdir, "stderr.txt")).read()
-        assert "extends beyond end of contig" in err and "failed to parse line in GTF file" in err and "CDS record has unknown transcript ID" in err
-        assert seed != 32 or "appears to be non-unique" in err
+        w = out[seed] = worldutil.reference_world(prefix, os.path.join(d, "oracle"))
+        assert w.stderr_has("extends beyond end of contig") and w.stderr_has("failed to parse line in GTF file") and w.stderr_has("CDS record has unknown transcript ID")
+        assert seed != 32 or w.stderr_has("appears to be non-unique")
     return out
 
 

@@ -1,5 +1,11 @@
-"""Test infrastructure: synthetic worlds, oracle runs, and conversion of oracle dumps into C-ABI inputs."""
-import os, subprocess, hashlib, json
+"""Test infrastructure: synthetic worlds, the reference's results on them, and conversion of oracle dumps into C-ABI inputs.
+
+The tests compare the product with the unmodified reference. What they compare against is committed in tests/golden/reference_runs.json:
+for every reference run the suite makes, keyed by the bytes of its input files and its arguments, the exit code, the ERROR lines, SHA-256
+digests of both output files and the digests / values of the stage dumps the tests look at. The suite reads that record and never needs the
+reference. Where the reference is built (oracle/_ref/arriba, see oracle/Makefile), `ARB_RECORD_REFERENCE=1 pytest -m "not gpu" tests` runs it
+instead and writes the record again; the CPU tests then check the product against the fresh runs while they record them."""
+import atexit, os, subprocess, hashlib, json, shutil, tempfile
 import numpy as np
 import arbdump
 from arriba_b200 import _build
@@ -9,6 +15,74 @@ INTERESTING = set([str(i) for i in range(1, 23)] + ["X", "Y"])
 
 # small, feature-dense default world (seconds for the oracle)
 SMALL = dict(scale=0.001, genes=400, breakpoints=200, fragments=20000, read_length=101)
+
+RECORD_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_runs.json")
+RECORDING = os.environ.get("ARB_RECORD_REFERENCE") == "1"
+
+
+def digest(a):
+    """SHA-256 (80 bits) of an array's values, independent of its integer width; floats by their bit patterns."""
+    a = np.asarray(a)
+    if a.dtype.kind == "f":
+        a = a.view(np.uint32 if a.itemsize == 4 else np.uint64)
+    return hashlib.sha256(np.ascontiguousarray(a.astype(np.int64)).ravel().tobytes()).hexdigest()[:20]
+
+
+def file_digest(path):
+    h = hashlib.sha256()
+    with open(path, "rb") as f:
+        for block in iter(lambda: f.read(1 << 22), b""):
+            h.update(block)
+    return h.hexdigest()
+
+
+class _Record:
+    """tests/golden/reference_runs.json: run key -> {fact name: value}. Recording rewrites it with the runs this session made."""
+    def __init__(self):
+        self.runs = None; self.fresh = {}
+
+    def get(self, key):
+        if RECORDING:
+            if not self.fresh:
+                atexit.register(self.save)
+            return self.fresh.setdefault(key, {})
+        if self.runs is None:
+            self.runs = json.load(open(RECORD_PATH)) if os.path.exists(RECORD_PATH) else {}
+        if key not in self.runs:
+            raise KeyError("no recorded reference run for these inputs (%s); record one with ARB_RECORD_REFERENCE=1 where oracle/_ref/arriba is built" % key)
+        return self.runs[key]
+
+    def save(self):
+        old = json.load(open(RECORD_PATH)) if os.path.exists(RECORD_PATH) else {}
+        old.update(self.fresh)
+        with open(RECORD_PATH, "w") as f:
+            json.dump(old, f, indent=0, sort_keys=True, separators=(",", ":"))
+            f.write("\n")
+
+
+RECORD = _Record()
+
+
+def run_key(files, args, kind="run"):
+    h = hashlib.sha256(json.dumps([kind, list(args)]).encode())
+    for path in files:
+        h.update(file_digest(path).encode())
+    return h.hexdigest()[:24]
+
+
+def reference_cli(bam, gtf, fa, args, det_alloc=False):
+    """The reference's command line on these files: (exit code, its ERROR lines, {output file: sha256} when it succeeded)."""
+    rec = RECORD.get(run_key((bam, gtf, fa), args, "cli"))
+    if "rc" not in rec:
+        if not RECORDING:
+            raise KeyError("incomplete reference record")
+        with tempfile.TemporaryDirectory() as d:
+            env = dict(os.environ, ARB_DET_ALLOC="1") if det_alloc else None
+            r = subprocess.run([_build.build_oracle(), "-x", bam, "-g", gtf, "-a", fa, "-o", d + "/o.tsv", "-O", d + "/d.tsv"] + list(args),
+                               capture_output=True, text=True, env=env, timeout=900)
+            rec["rc"] = r.returncode; rec["errors"] = [l for l in r.stderr.split("\n") if l.startswith("ERROR")]
+            rec["sha"] = {"fusions.tsv": file_digest(d + "/o.tsv"), "fusions.discarded.tsv": file_digest(d + "/d.tsv")} if r.returncode == 0 else None
+    return rec["rc"], rec["errors"], rec["sha"]
 
 
 def run_synth(prefix, seed=0xA881BA, scale=0.001, genes=400, breakpoints=200, fragments=20000, read_length=101, extra=()):
@@ -40,9 +114,39 @@ def run_oracle(prefix, outdir, dump=True, det_alloc=True, args=("-f", "blacklist
 
 
 class World:
-    def __init__(self, prefix, outdir):
+    """The input files at `prefix` and the reference's run on them (with stage dumps). `fact(name, compute)` is what the tests compare
+    against: recorded, or, while recording, compute(self) over the oracle's dumps and output files in `outdir`."""
+    def __init__(self, prefix, outdir=None, args=("-f", "blacklist")):
         self.prefix = prefix; self.outdir = outdir
+        self.key = run_key((prefix + ".bam", prefix + ".gtf", prefix + ".fa"), args)
         self._dumps = None; self._fasta = None
+
+    def fact(self, name, compute):
+        rec = RECORD.get(self.key)
+        if name not in rec:
+            if not RECORDING:
+                raise KeyError("the reference record of %s has no %r; record it with ARB_RECORD_REFERENCE=1 where oracle/_ref/arriba is built" % (self.key, name))
+            rec[name] = compute(self)
+        return rec[name]
+
+    def stage_digest(self, name, column, occurrence=0):
+        return self.fact("%s/%d/%s" % (name, occurrence, column), lambda w: digest(w.stage(name, occurrence)[column]))
+
+    def stage_scalar(self, name, column, occurrence=0):
+        return self.fact("%s/%d/%s[0]" % (name, occurrence, column), lambda w: w.stage(name, occurrence)[column][0].item())
+
+    def output_digest(self, filename):
+        return self.fact("sha256/" + filename, lambda w: file_digest(os.path.join(w.outdir, filename)))
+
+    def output_lines(self, filename):
+        return self.fact("lines/" + filename, lambda w: len(open(os.path.join(w.outdir, filename)).read().split("\n")))
+
+    def stderr_has(self, phrase):
+        return self.fact("stderr/" + phrase, lambda w: phrase in open(os.path.join(w.outdir, "stderr.txt")).read())
+
+    def same_output(self, filename, path):
+        """the file at `path` is byte for byte the reference's `filename`"""
+        return file_digest(path) == self.output_digest(filename)
 
     @property
     def dumps(self):
@@ -60,6 +164,13 @@ class World:
         return self._fasta
 
 
+def reference_world(prefix, outdir, args=("-f", "blacklist")):
+    """The reference's run on the files at `prefix` (run only while recording)."""
+    if RECORDING:
+        run_oracle(prefix, outdir, args=args)
+    return World(prefix, outdir, args)
+
+
 class WorldCache:
     def __init__(self, root):
         self.root = root; self.cache = {}
@@ -72,8 +183,7 @@ class WorldCache:
             prefix = os.path.join(d, "w")
             extra = params.pop("extra", ())
             run_synth(prefix, extra=extra, **params)
-            run_oracle(prefix, os.path.join(d, "oracle"), args=oracle_args)
-            self.cache[key] = World(prefix, os.path.join(d, "oracle"))
+            self.cache[key] = reference_world(prefix, os.path.join(d, "oracle"), oracle_args)
         return self.cache[key]
 
 
@@ -175,15 +285,56 @@ def annotation_from_dump(fl, n_contigs):
     return a
 
 
-def context_from_oracle(world, lib_path, device=0):
-    """Context loaded with the oracle's annotated fragments, annotation and the world's contigs."""
-    from arriba_b200 import lib
-    ctx = lib.Context(device, lib_path)
-    names, flags, seqs = contigs_from_world(world)
-    fl = world.stage("fragment_length")
-    n_contigs = max(len(names), int(fl["gene_contig"].max()) + 1)
-    assert n_contigs == len(names)
-    ctx.set_contigs(flags, seqs)
-    ctx.set_annotation(annotation_from_dump(fl, n_contigs))
-    ctx.push_chunk(chunk_from_dump(world.stage("annotated")))
-    return ctx
+def _segments(data, starts, counts):
+    """concatenation of data[starts[i]:starts[i] + counts[i]] over i"""
+    starts = np.asarray(starts, np.int64); counts = np.asarray(counts, np.int64)
+    total = int(counts.sum())
+    if total == 0:
+        return np.zeros(0, np.int64)
+    return np.asarray(data)[np.arange(total) + np.repeat(starts - (np.cumsum(counts) - counts), counts)]
+
+
+def fragment_digests(t, names, name_off, check_genes, check_pred):
+    """Digests of a fragment table in arb_soa_chunk layout (Pipeline.fragments() or chunk_from_dump()): the fields of the alignments that exist,
+    CIGARs, sequences and gene sets alignment by alignment, whatever offsets the variable-length parts sit at."""
+    n = int(t["n_fragments"])
+    valid = (t["n_aln"][None, :] > np.arange(3)[:, None]).ravel()
+    mask = 0b001011 | (0b000100 if check_genes else 0) | (0b100000 if check_pred else 0)
+    out = {"n": n, "names": digest(np.frombuffer(names, np.uint8)), "name_off": digest(name_off), "n_aln": digest(t["n_aln"]), "fflags": digest(t["fflags"])}
+    for k in ("contig", "start", "end", "cigar_cnt"):
+        out[k] = digest(t[k][valid])
+    out["aflags"] = digest(t["aflags"][valid] & mask)
+    if check_pred:   # the predicted strand only where it is not ambiguous
+        out["predicted_strand"] = digest(t["aflags"][valid & ((t["aflags"] & 32) == 0)] & 16)
+    out["cigar"] = digest(_segments(t["cigar"], t["cigar_off"][valid], t["cigar_cnt"][valid]))
+    v2 = valid[:2 * n]
+    lens = t["seq_len"][v2].astype(np.int64)
+    out["seq_len"] = digest(lens)
+    out["seq"] = digest(_segments(t["seq"], t["seq_off"][v2].astype(np.int64) * 16, (lens + 1) // 2))
+    if check_genes:
+        out["genes_cnt"] = digest(t["genes_cnt"][valid])
+        out["genes"] = digest(_segments(t["genes"], t["genes_off"][valid], t["genes_cnt"][valid]))
+    return out
+
+
+def frag_tables_equal(got, world, stage, check_genes, check_pred):
+    """got: Pipeline.fragments(); the reference's fragment table of dump stage `stage` (ingest / annotated)."""
+    def ref(w):
+        d = w.stage(stage)
+        return fragment_digests(chunk_from_dump(d), bytes(d["names"]), d["name_off"], check_genes, check_pred)
+    want = world.fact("fragments/%s/%d%d" % (stage, check_genes, check_pred), ref)
+    mine = fragment_digests(got, got["names_blob"], got["name_off"], check_genes, check_pred)
+    bad = [k for k in want if mine[k] != want[k]]
+    assert not bad, "fragment table differs from the reference's (%s) in %s" % (stage, bad)
+
+
+def front_end(world, lib_path, threads=4, device=0):
+    """Pipeline on the world's files up to the upload of the fragment table, whose annotated fragments are checked to be the reference's:
+    the device stages after it start from the reference's input."""
+    from arriba_b200 import lib as L
+    p = L.Pipeline(world.prefix + ".bam", world.prefix + ".gtf", world.prefix + ".fa", threads=threads, device=device, lib_path=lib_path)
+    for s in (L.STEP_LOAD_REFERENCE, L.STEP_INGEST, L.STEP_ANNOTATE):
+        p.step(s)
+    frag_tables_equal(p.fragments(), world, "annotated", check_genes=True, check_pred=True)
+    p.step(L.STEP_UPLOAD)
+    return p
