@@ -17,7 +17,7 @@ SYNTH_BIN = os.path.join(ROOT, "build", "synth")
 ORACLE_BIN = os.path.join(ROOT, "oracle", "_ref", "arriba")
 REFERENCE = "/root/reference/source"
 
-CU_SOURCES = ["prims.cu", "engine.cu", "bamscan.cu", "annotate.cu", "fusions.cu", "events.cu", "rows.cu", "consensus.cu", "mismap.cu", "exchange.cu", "capi.cu", "selftest.cu"]
+CU_SOURCES = ["prims.cu", "engine.cu", "bamscan.cu", "fragtable.cu", "annotate.cu", "fusions.cu", "events.cu", "rows.cu", "consensus.cu", "mismap.cu", "exchange.cu", "capi.cu", "selftest.cu"]
 CPP_SOURCES = ["mismatch_table.cpp", "host/refdata.cpp", "host/ingest.cpp", "host/annotate.cpp", "host/viral.cpp", "host/pipeline.cpp", "host/events.cpp", "host/output.cpp", "host/shard.cpp", "host/host_capi.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--fmad=false",
               "-Xcompiler", "-fPIC,-O2,-Wall,-Wno-unused-function", "-Xptxas", "-v"]

@@ -91,6 +91,11 @@ int arb_push_chunk_end(arb_ctx* ctx, const arb_soa_chunk* c) { ARB_API_BEGIN(ctx
 int arb_bam_scan(arb_ctx* ctx, const uint8_t* chunk, uint64_t bytes, uint64_t first, int32_t n_ref, uint32_t n_lists, uint64_t* consumed, uint32_t* n_records, uint32_t* list_begin, uint32_t* record_offsets, uint32_t* malformed) {
 	ARB_API_BEGIN(ctx) u64 c = 0; ctx->e.bam_scan(chunk, bytes, first, n_ref, n_lists, &c, n_records, list_begin, record_offsets, malformed); *consumed = c; ARB_API_END(ctx)
 }
+int arb_build_fragment_table(arb_ctx* ctx, const arb_ingest_pool* pools, uint32_t n_pools, arb_fragment_table_sizes* sizes) {
+	ARB_API_BEGIN(ctx) if (!sizes) throw arb_error("arb_build_fragment_table: sizes is NULL"); memset(sizes, 0, sizeof(*sizes)); ctx->e.build_fragment_table(pools, n_pools, *sizes); ARB_API_END(ctx)
+}
+uint32_t arb_fragment_table_tie_rounds(arb_ctx* ctx) { return ctx ? ctx->e.tie_rounds : 0; }
+int arb_get_fragment_table(arb_ctx* ctx, const arb_fragment_columns* out) { ARB_API_BEGIN(ctx) if (!out) throw arb_error("arb_get_fragment_table: out is NULL"); ctx->e.get_fragment_table(*out); ARB_API_END(ctx) }
 int arb_annotate_pass1(arb_ctx* ctx, const uint8_t* aflags, int32_t strandedness, uint32_t* n_dummy) { ARB_API_BEGIN(ctx) const uint32_t k = ctx->e.annotate_pass1(aflags, strandedness); if (n_dummy) *n_dummy = k; ARB_API_END(ctx) }
 int arb_get_dummy_genes(arb_ctx* ctx, uint16_t* contig, int32_t* start, int32_t* end) { ARB_API_BEGIN(ctx) ctx->e.get_dummy_genes(contig, start, end); ARB_API_END(ctx) }
 int arb_annotate_pass2(arb_ctx* ctx, uint64_t* n_gene_ids) { ARB_API_BEGIN(ctx) const uint64_t k = ctx->e.annotate_pass2(); if (n_gene_ids) *n_gene_ids = k; ARB_API_END(ctx) }

@@ -14,7 +14,7 @@ void default_params(arb_params& p) { // options.cpp:71-107
 	p.max_mismapper_fraction = 0.8f; p.max_homolog_identity = 0.3f;
 }
 
-engine::engine(): row_max_itd_length(0), has_row_texts(false), row_text_bytes(0), kmer_block_shift(0), kmer_blocks(0), coverage_contigs(0), work_part(0), work_parts(1), mismap_items_total(0), mismap_ms_part(0), n_splice_sites(0), annot_pool_cap(0), n_dummy(0), n_gene_entries(0), push_cigar_ops(0), cascade_smem_bytes(0), cascade_resident_blocks(0), device(0), table_n(0), table_k(0), has_contigs(false), has_annotation(false), filters_done(false), merge_log_n(0), kmer_index_contigs(0), kmer_indexed(0), has_splice_sites(false) {
+engine::engine(): ft_n_name_bytes(0), tie_rounds(0), row_max_itd_length(0), has_row_texts(false), row_text_bytes(0), kmer_block_shift(0), kmer_blocks(0), coverage_contigs(0), work_part(0), work_parts(1), mismap_items_total(0), mismap_ms_part(0), n_splice_sites(0), annot_pool_cap(0), n_dummy(0), n_gene_entries(0), push_cigar_ops(0), cascade_smem_bytes(0), cascade_resident_blocks(0), device(0), table_n(0), table_k(0), has_contigs(false), has_annotation(false), filters_done(false), merge_log_n(0), kmer_index_contigs(0), kmer_indexed(0), has_splice_sites(false) {
 	default_params(params);
 	memset(&timings, 0, sizeof(timings));
 	cons_rows = 0; cons_seq_bytes = cons_pos_count = cons_clip_bytes = 0;
@@ -178,11 +178,18 @@ void engine::push_chunk_begin(const arb_soa_chunk& c) {
 	const exec_ctx& cx = copy_ex;
 	stage_timer t_h2d(cx);
 	frags.n_aln.upload(cx, c.n_aln, n); frags.fflags.upload(cx, c.fflags, n); frags.filter.upload(cx, c.filter, n);
-	frags.early.ensure(n); frags.swapped.ensure(n); frags.swapped.zero(cx, n);
 	frags.contig.upload(cx, c.contig, 3 * (size_t) n); frags.start.upload(cx, c.start, 3 * (size_t) n); frags.end.upload(cx, c.end, 3 * (size_t) n);
 	frags.cigar_off.upload(cx, c.cigar_off, 3 * (size_t) n); frags.cigar_cnt.upload(cx, c.cigar_cnt, 3 * (size_t) n);
 	frags.seq_off.upload(cx, c.seq_off, 2 * (size_t) n); frags.seq_len.upload(cx, c.seq_len, 2 * (size_t) n);
 	frags.cigar.upload(cx, c.cigar, c.n_cigar); frags.seq.upload(cx, c.seq, c.n_seq_bytes);
+	table_resident(cx, c.n_cigar, c.n_seq_bytes);
+	timings.h2d_ms = t_h2d.stop(); // waits for part one: the caller's annotation takes far longer than the copy, and the timing stays a pure copy time
+	timings.h2d_bytes = (u64) n * 3 + (u64) n * 3 * (2 + 4 + 4 + 4 + 2) + (u64) n * 2 * (4 + 2) + c.n_cigar * 4 + c.n_seq_bytes;
+}
+
+void engine::table_resident(const exec_ctx& cx, u64 n_cigar, u64 n_seq_bytes) {
+	const u32 n = frags.n;
+	frags.early.ensure(n); frags.swapped.ensure(n); frags.swapped.zero(cx, n);
 	// statistics of the chunk, taken on the device behind the copies (a pass over four columns: serial on the host it cost a tenth of a second per 10 M
 	// fragments): longest sequence, bases, alignments, and whether the sequence pool has the canonical layout (what ingest writes: sequences in fragment
 	// order, slot 0 then slot 1, back to back in 16-byte units -- the sequence kernel then stages a tile of fragments with one bulk copy)
@@ -192,11 +199,9 @@ void engine::push_chunk_begin(const arb_soa_chunk& c) {
 	u64 st[4] = {0, 0, 0, 0};
 	chunk_stats.download(cx, st, 4);
 	frags.max_seq_len = (u32) st[0];
-	frags.n_seq_bytes = c.n_seq_bytes;
-	frags.canonical_seq_layout = n > 0 && c.n_seq_bytes % 16 == 0 && st[3] == 0;
-	push_alignments = st[2]; push_bases = st[1]; push_cigar_ops = c.n_cigar;
-	timings.h2d_ms = t_h2d.stop(); // waits for part one: the caller's annotation takes far longer than the copy, and the timing stays a pure copy time
-	timings.h2d_bytes = (u64) n * 3 + (u64) n * 3 * (2 + 4 + 4 + 4 + 2) + (u64) n * 2 * (4 + 2) + c.n_cigar * 4 + c.n_seq_bytes;
+	frags.n_seq_bytes = n_seq_bytes;
+	frags.canonical_seq_layout = n > 0 && n_seq_bytes % 16 == 0 && st[3] == 0;
+	push_alignments = st[2]; push_bases = st[1]; push_cigar_ops = n_cigar;
 	push_open = true;
 	filters_done = false;
 	cands.n = 0;

@@ -104,6 +104,11 @@ public:
 	void push_chunk(const arb_soa_chunk& c) { push_chunk_begin(c); push_chunk_end(c); }
 	void push_chunk_begin(const arb_soa_chunk& c); // everything but the annotation columns (aflags, gene sets), asynchronously on the copy stream
 	void push_chunk_end(const arb_soa_chunk& c);   // the annotation columns; returns when the whole table is resident
+	// the fragment table built on the device from the ingest workers' pools (fragtable.cu): resident afterwards as after push_chunk_begin
+	void build_fragment_table(const arb_ingest_pool* pools, u32 n_pools, arb_fragment_table_sizes& sizes); void get_fragment_table(const arb_fragment_columns& out);
+	dbuf<char> ft_names, ft_out_names; dbuf<u32> ft_cigars, ft_frag_base; dbuf<u8> ft_seqs; dbuf<arb_pool_alignment> ft_alns; dbuf<arb_pool_fragment> ft_frags; dbuf<u64> ft_bases, ft_out_name_off;
+	u64 ft_n_name_bytes; u32 tie_rounds;
+	void table_resident(const exec_ctx& cx, u64 n_cigar, u64 n_seq_bytes); // bookkeeping once the ingest columns of frags.n fragments are on the device
 	// device-side annotation of the resident chunk (annotate.cu): between the two passes the gene sets live in fixed rows + a pool
 	u32 annotate_pass1(const u8* aflags, int strandedness); void get_dummy_genes(u16* contig, i32* start, i32* end); u64 annotate_pass2();
 	void get_annotation_columns(u8* aflags, u32* genes_off, u16* genes_cnt, u32* genes);

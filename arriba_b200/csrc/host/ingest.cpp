@@ -1,6 +1,6 @@
 // ingest.cpp -- see ingest.h. BGZF blocks are inflated in parallel, records are sharded by read name over worker threads
 // (every alignment of a read name is handled by the same worker, so mate collation and "first insertion wins" stay local),
-// and the fragments are finally ordered by name, which is the order every later stage relies on.
+// and the fragments are finally ordered by name on the device (csrc/fragtable.cu), which is the order every later stage relies on.
 #include "ingest.h"
 #include "../../../include/arriba_b200.h"
 #include <set>
@@ -179,30 +179,28 @@ static bool clipped_at_correct_end(const rec_t& r) {
 }
 
 // ------------------------------------------------------------------------------------------- per-worker fragment store
-struct aln_build { u8 supplementary, first_in_pair, forward; u16 contig; i32 start, end; u32 cigar_off, cigar_cnt; u64 seq_off; u32 seq_len; i32 next; };
-struct frag_build { u64 name_off; u32 name_len; i32 head, tail; u32 count; u8 single_end, duplicate; };
+// the records of the pools that arb_build_fragment_table turns into the fragment table on the device
+typedef arb_pool_alignment aln_build;
+typedef arb_pool_fragment frag_build;
 
-struct final_frag { u32 worker; u32 frag; u64 prefix0, prefix1; };
-struct name_ref { const char* p; u32 len; };
 struct name_hash { size_t operator()(const std::string& s) const { u64 h = 1469598103934665603ULL; for (size_t i = 0; i < s.size(); ++i) { h ^= (u8) s[i]; h *= 1099511628211ULL; } return (size_t) h; } };
 
 struct worker {
 	refdata* ref; const ingest_options* opt; const std::vector<u16>* tid_to_contig; const std::vector<u8>* interesting_contig; const std::vector<u8>* viral_contig;
 	annot_view an;
-	std::vector<char> names; std::vector<u32> cigars; std::vector<u8> seqs; std::vector<aln_build> alns; std::vector<frag_build> frags;
-	std::vector<aln_build> norm_alns; std::vector<u32> norm_cigars; // the fragments' alignments after slot normalisation, contiguous per fragment
+	// append-only pools, page-locked (host blocks of the CUDA library): they are copied to the device as they are when the record loop ends
+	column<char> names; column<u32> cigars; column<u8> seqs; column<aln_build> alns; column<frag_build> frags;
 	std::vector<u32> name_slots; // open-addressing index of `frags` by name: fragment id + 1, 0 = empty; names are compared in the `names` pool
 	std::unordered_map<std::string, std::vector<u8>, name_hash> pending; // first mate of a proper pair, waiting for the second
 	coverage_windows* cov; // shared by all workers: saturating counters and flags are updated atomically, the result does not depend on the order
 	u64 mapped_reads, malformed, missing_hi, records; std::vector<u64> viral_reads; bool no_chimeric;
 	std::string key, clip_chars, waiting_key; const u8* waiting_ptr; u32 waiting_size; u32 last_fragment;
 	void park_waiting() { if (waiting_ptr) { pending.emplace(waiting_key, std::vector<u8>(waiting_ptr, waiting_ptr + waiting_size)); waiting_ptr = NULL; } } // before the chunk buffer is recycled
-	std::vector<final_frag> keep; // the fragments that survive slot normalisation, with their name prefixes
 	worker(): cov(NULL), waiting_ptr(NULL), waiting_size(0), last_fragment(0xFFFFFFFFu), mapped_reads(0), malformed(0), missing_hi(0), records(0), no_chimeric(true), key_hash_hint(0) {}
 	// A worker's pools are gigabytes that a sample touches for the first time page by page (a tenth of the ingest's CPU time went into those faults, tools/hostprof
 	// on the GPU box): the workers of a finished sample are kept for the next one -- contents dropped, memory kept (arb_release_host_memory gives it back).
 	void recycle() {
-		names.clear(); cigars.clear(); seqs.clear(); alns.clear(); frags.clear(); norm_alns.clear(); norm_cigars.clear(); keep.clear(); pending.clear(); viral_reads.clear();
+		names.clear(); cigars.clear(); seqs.clear(); alns.clear(); frags.clear(); pending.clear(); viral_reads.clear();
 		std::fill(name_slots.begin(), name_slots.end(), 0u);
 		ref = NULL; opt = NULL; tid_to_contig = NULL; interesting_contig = NULL; viral_contig = NULL; cov = NULL;
 		mapped_reads = malformed = missing_hi = records = 0; no_chimeric = true; waiting_ptr = NULL; waiting_size = 0; last_fragment = 0xFFFFFFFFu; key_hash_hint = 0;
@@ -283,7 +281,7 @@ struct worker {
 		name_slots.swap(bigger);
 	}
 	// After the first chunk the final size of every pool can be estimated from the share of the file seen so far. Growing a pool by doubling copies it again
-	// and again into fresh pages (gigabytes per worker on a large sample); one reservation up front is virtual memory until it is used. A hint only: the
+	// and again into fresh pages (gigabytes per worker on a large sample); one reservation up front avoids that (it is page-locked and kept for the next sample). A hint only: the
 	// pools still grow by themselves where the estimate falls short; `cap_bytes` bounds what one pool may reserve.
 	void reserve_ahead(double factor, size_t cap_bytes) {
 		auto grow = [&](auto& v) {
@@ -729,67 +727,6 @@ template <class F> static void parallel_for(int threads, size_t n, F f) { // f(t
 	for (int t = 0; t < threads; ++t) if (!errors[t].empty()) fail(errors[t]);
 }
 
-// ------------------------------------------------------------------------------------------- slot normalisation
-// Brings a fragment's alignments into the canonical slots (MATE1, MATE2/SPLIT_READ, SUPPLEMENTARY) or rejects it
-// (read_chimeric_alignments.cpp:340-373 disjoin_split_read_segments, :377-506 remove_malformed_alignments).
-struct norm_aln { aln_build a; std::vector<u32> cigar; };
-static u32 clip_of(const norm_aln& x, bool front) { const u32 c = front ? x.cigar.front() : x.cigar.back(); const u32 o = c & 15; return (o == C_S || o == C_H) ? c >> 4 : 0; }
-
-static bool disjoin_segments(norm_aln& split, norm_aln& supp) {
-	const u32 clipped_split = split.a.forward ? clip_of(split, true) : clip_of(split, false);
-	const u32 clipped_supp = supp.a.forward ? clip_of(supp, false) : clip_of(supp, true);
-	const int overlap = (int) split.a.seq_len - (int) clipped_split - (int) clipped_supp;
-	if (overlap <= 0) return true;
-	const u32 clipped_op = supp.a.forward ? (u32) supp.cigar.size() - 1 : 0;
-	const u32 matching_op = supp.a.forward ? clipped_op - 1 : 1;
-	if (supp.cigar.size() < 2 || (supp.cigar[matching_op] & 15) != C_M || (int) (supp.cigar[matching_op] >> 4) < overlap + 10) return false;
-	supp.cigar[clipped_op] = ((supp.cigar[clipped_op] >> 4) + overlap) << 4 | (supp.cigar[clipped_op] & 15);
-	supp.cigar[matching_op] = ((supp.cigar[matching_op] >> 4) - overlap) << 4 | (supp.cigar[matching_op] & 15);
-	if (supp.a.forward) supp.a.end -= overlap; else supp.a.start += overlap;
-	return true;
-}
-
-static bool normalise_fragment(std::vector<norm_aln>& m, bool single_end) {
-	if (single_end) {
-		if (!(m.size() == 2 && (m[0].a.supplementary != m[1].a.supplementary))) return false;
-		// the longer anchor becomes the split read; it is duplicated into the MATE1 slot to imitate paired-end data
-		if (m[0].a.end - m[0].a.start > m[1].a.end - m[1].a.start) { m.push_back(m[1]); m[1] = m[0]; }
-		else { m.push_back(m[0]); m[0] = m[1]; }
-		// sequence: MATE1 and SPLIT_READ carry it, SUPPLEMENTARY does not
-		if (!m[0].a.supplementary) { m[1].a.seq_off = m[0].a.seq_off; m[1].a.seq_len = m[0].a.seq_len; }
-		else if (!m[1].a.supplementary) { m[0].a.seq_off = m[1].a.seq_off; m[0].a.seq_len = m[1].a.seq_len; }
-		else { m[0].a.seq_off = m[1].a.seq_off = m[2].a.seq_off; m[0].a.seq_len = m[1].a.seq_len = m[2].a.seq_len; }
-		m[2].a.seq_len = 0;
-		for (int s = 0; s < 2; ++s) {
-			if ((m[s].cigar.front() & 15) == C_H) m[s].cigar.front() = (m[s].cigar.front() >> 4) << 4 | C_S;
-			if ((m[s].cigar.back() & 15) == C_H) {
-				// the reference takes the length for SPLIT_READ's last op from MATE1's CIGAR at the same index (read_chimeric_alignments.cpp:415)
-				const u32 len = s == 0 ? m[0].cigar.back() >> 4 : (m[1].cigar.size() - 1 < m[0].cigar.size() ? m[0].cigar[m[1].cigar.size() - 1] >> 4 : 0);
-				m[s].cigar.back() = len << 4 | C_S;
-			}
-		}
-		m[2].a.supplementary = 1; m[0].a.supplementary = 0; m[1].a.supplementary = 0;
-		const bool same = m[1].a.forward == m[2].a.forward;
-		const u32 len = m[1].a.seq_len;
-		const u32 lhs = len - clip_of(m[1], true) - (same ? clip_of(m[2], false) : clip_of(m[2], true));
-		const u32 rhs = len - clip_of(m[1], false) - (same ? clip_of(m[2], true) : clip_of(m[2], false));
-		const bool flip = lhs < rhs ? (m[1].a.forward != 0) : (m[1].a.forward == 0);
-		if (flip) m[0].a.forward = !m[0].a.forward; else { m[1].a.forward = !m[1].a.forward; m[2].a.forward = !m[2].a.forward; }
-		m[0].a.first_in_pair = !flip; m[1].a.first_in_pair = flip; m[2].a.first_in_pair = flip;
-		if (!disjoin_segments(m[1], m[2])) return false;
-	} else if (m.size() == 3) {
-		if (m[0].a.supplementary) std::swap(m[0], m[2]); else if (m[1].a.supplementary) std::swap(m[1], m[2]);
-		if (m[1].a.first_in_pair != m[2].a.first_in_pair) std::swap(m[0], m[1]);
-		if (m[0].a.supplementary || m[1].a.supplementary || !m[2].a.supplementary) return false;
-		if (m[0].a.contig != m[1].a.contig || m[0].a.forward == m[1].a.forward) return false;
-		if (!disjoin_segments(m[1], m[2])) return false;
-	} else if (m.size() == 2) {
-		if (m[0].a.supplementary || m[1].a.supplementary) return false;
-	} else return false;
-	for (int s = 0; s < 2; ++s) if ((m[s].cigar.front() & 15) == C_H || (m[s].cigar.back() & 15) == C_H) return false; // anchors need their full sequence
-	return true;
-}
-
 // ------------------------------------------------------------------------------------------- driver
 frag_view fragment_table::view() {
 	frag_view v;
@@ -956,173 +893,39 @@ void read_chimeric_alignments(const std::string& bam_path, refdata& ref, const i
 	lap("merge by-products");
 	if (stats.mapped_reads == 0) fail("no normal reads found");
 
-	// ---- slot normalisation, rejection of malformed fragments ----
-	std::vector<u64> malformed_by_worker(T, 0);
-	parallel_for(T, (size_t) T, [&](int, size_t lo, size_t hi) {
-		for (size_t t = lo; t < hi; ++t) {
-			worker& w = workers[t];
-			std::vector<norm_aln> m;
-			const size_t n_frags = w.frags.size(); // fixed: only alignments and CIGARs are appended below
-			w.keep.reserve(n_frags);
-			w.norm_alns.reserve(w.alns.size()); w.norm_cigars.reserve(w.cigars.size()); advise_huge(w.norm_alns.data(), w.norm_alns.capacity() * sizeof(aln_build)); advise_huge(w.norm_cigars.data(), w.norm_cigars.capacity() * sizeof(u32)); // normalisation drops alignments, it never adds one: no regrowth, and the parsed pools are not copied
-			for (size_t f = 0; f < n_frags; ++f) {
-				// a fragment's alignments were stored as its records arrived, far apart: the chain of the fragments a few steps ahead is requested early
-				if (f + 12 < n_frags && w.frags[f + 12].head >= 0) { __builtin_prefetch(&w.alns[w.frags[f + 12].head]); __builtin_prefetch(w.names.data() + w.frags[f + 12].name_off); }
-				if (f + 8 < n_frags && w.frags[f + 8].head >= 0) { const aln_build& a = w.alns[w.frags[f + 8].head]; __builtin_prefetch(&w.cigars[a.cigar_off]); if (a.next >= 0) __builtin_prefetch(&w.alns[a.next]); }
-				if (f + 4 < n_frags && w.frags[f + 4].head >= 0) { const i32 second = w.alns[w.frags[f + 4].head].next; if (second >= 0) { const aln_build& a = w.alns[second]; __builtin_prefetch(&w.cigars[a.cigar_off]); if (a.next >= 0) __builtin_prefetch(&w.alns[a.next]); } }
-				frag_build& fb = w.frags[f];
-				size_t count = 0; // the scratch alignments keep their CIGAR storage from fragment to fragment
-				for (i32 a = fb.head; a >= 0; a = w.alns[a].next, ++count) {
-					if (m.size() <= count) m.resize(count + 1);
-					m[count].a = w.alns[a]; m[count].cigar.assign(w.cigars.begin() + m[count].a.cigar_off, w.cigars.begin() + m[count].a.cigar_off + m[count].a.cigar_cnt);
-				}
-				m.resize(count);
-				if (!normalise_fragment(m, fb.single_end)) { ++malformed_by_worker[t]; fb.count = 0; continue; }
-				// write the normalised alignments back (fresh CIGAR storage; slots become contiguous)
-				fb.head = (i32) w.norm_alns.size(); fb.count = (u32) m.size();
-				for (size_t s = 0; s < m.size(); ++s) {
-					m[s].a.cigar_off = (u32) w.norm_cigars.size(); m[s].a.cigar_cnt = (u32) m[s].cigar.size();
-					w.norm_cigars.insert(w.norm_cigars.end(), m[s].cigar.begin(), m[s].cigar.end());
-					w.norm_alns.push_back(m[s].a);
-				}
-				final_frag ff; ff.worker = (u32) t; ff.frag = (u32) f; ff.prefix0 = ff.prefix1 = 0;
-				const char* nm = w.names.data() + fb.name_off;
-				for (u32 k = 0; k < 16 && k < fb.name_len; ++k) { u64& dst = k < 8 ? ff.prefix0 : ff.prefix1; dst |= (u64) (u8) nm[k] << (56 - 8 * (k & 7)); }
-				w.keep.push_back(ff);
-			}
-		}
-	});
-	lap("normalise slots");
-	for (int t = 0; t < T; ++t) stats.malformed += malformed_by_worker[t];
+	// ---- the fragment table: slot normalisation, name order, columns and multimapper flags, on the device (csrc/fragtable.cu) ----
+	std::vector<arb_ingest_pool> pools(T);
+	for (int t = 0; t < T; ++t) {
+		const worker& w = workers[t]; arb_ingest_pool& q = pools[t];
+		q.names = w.names.data(); q.n_name_bytes = w.names.size(); q.cigars = w.cigars.data(); q.n_cigars = w.cigars.size(); q.seqs = w.seqs.data(); q.n_seq_bytes = w.seqs.size();
+		q.alns = w.alns.data(); q.n_alns = w.alns.size(); q.frags = w.frags.data(); q.n_frags = (u32) w.frags.size();
+	}
+	arb_fragment_table_sizes sz;
+	if (arb_build_fragment_table(opt.scan_ctx, pools.data(), (u32) T, &sz) != 0) fail(arb_last_error(opt.scan_ctx));
+	if (trace) fprintf(stderr, "[ingest]   of which pools -> device %.1f ms, whole device build %.1f ms, %u name-sort rounds past the first 16 bytes\n", sz.upload_ms, sz.build_ms, sz.tie_rounds);
+	lap("fragment table (device)");
+	stats.malformed += sz.n_rejected;
 	if (stats.malformed > 0) std::cerr << "WARNING: " << stats.malformed << " SAM records were malformed and ignored" << std::endl;
 	if (stats.no_chimeric_reads) fail("no split reads or discordant mates found (STAR must either be run with '--chimOutType WithinBAM' or the file 'Chimeric.out.sam' must be passed to Arriba via the argument -c)");
 	if (stats.missing_hi_tag > 0) std::cerr << "WARNING: " << stats.missing_hi_tag << " secondary alignments lack the 'HI' tag and were ignored (STAR must be run with '--outSAMattributes HI' for Arriba to make use of multi-mapping reads for fusion detection)" << std::endl;
 
-	// ---- name order: std::string::compare semantics == unsigned byte-wise comparison, shorter string first on a common prefix ----
-	std::vector<final_frag, default_init_allocator<final_frag> > order;
-	{ // every worker's list goes to its own stretch of the table, copied (and first touched) by its own thread
-		std::vector<size_t> at(T + 1, 0); for (int t = 0; t < T; ++t) at[t + 1] = at[t] + workers[t].keep.size();
-		order.resize(at[T]);
-		parallel_for(T, (size_t) T, [&](int, size_t lo, size_t hi) { for (size_t t = lo; t < hi; ++t) { std::copy(workers[t].keep.begin(), workers[t].keep.end(), order.begin() + at[t]); workers[t].keep.clear(); } });
-	}
-	auto name_less = [&](const final_frag& a, const final_frag& b) {
-		if (a.prefix0 != b.prefix0) return a.prefix0 < b.prefix0;
-		if (a.prefix1 != b.prefix1) return a.prefix1 < b.prefix1;
-		const frag_build& fa = workers[a.worker].frags[a.frag]; const frag_build& fb = workers[b.worker].frags[b.frag];
-		const u32 n = std::min(fa.name_len, fb.name_len);
-		const int c = n > 16 ? memcmp(workers[a.worker].names.data() + fa.name_off + 16, workers[b.worker].names.data() + fb.name_off + 16, n - 16) : 0;
-		if (c != 0) return c < 0;
-		return fa.name_len < fb.name_len;
-	};
-	{ // parallel sort: T sorted slices, then rounds of pairwise merges; every merge is itself cut into independent pieces (by output rank), so all threads
-	  // stay busy down to the last round, where one merge spans the whole table
-		const size_t n = order.size();
-		std::vector<size_t> cut(T + 1); for (int t = 0; t <= T; ++t) cut[t] = n * t / T;
-		parallel_for(T, (size_t) T, [&](int, size_t lo, size_t hi) { for (size_t t = lo; t < hi; ++t) std::sort(order.begin() + cut[t], order.begin() + cut[t + 1], name_less); });
-		std::vector<final_frag, default_init_allocator<final_frag> > spare(T > 1 ? n : 0);
-		final_frag* src = order.data(); final_frag* dst = spare.data();
-		// how many elements of A = src[a, m) precede output rank r of merge(A, B = src[m, b)); equal keys take A first (names are unique anyway)
-		auto split = [&](const final_frag* A, size_t nA, const final_frag* B, size_t nB, size_t r) {
-			size_t lo = r > nB ? r - nB : 0, hi = std::min(r, nA);
-			while (lo < hi) { const size_t i = lo + (hi - lo) / 2, j = r - i; if (j == 0 || name_less(B[j - 1], A[i])) hi = i; else lo = i + 1; }
-			return lo;
-		};
-		for (int width = 1; width < T; width *= 2) {
-			std::vector<std::thread> pool;
-			for (int t = 0; t < T; t += 2 * width) {
-				const size_t a = cut[t], m = cut[std::min(T, t + width)], b = cut[std::min(T, t + 2 * width)];
-				const int parts = std::min(T - t, 2 * width); // as many threads as the merge has slices
-				for (int k = 0; k < parts; ++k) pool.emplace_back([&, a, m, b, k, parts]() {
-					const final_frag* A = src + a; const final_frag* B = src + m; const size_t nA = m - a, nB = b - m;
-					const size_t r0 = (b - a) * k / parts, r1 = (b - a) * (k + 1) / parts;
-					const size_t i0 = split(A, nA, B, nB, r0), i1 = split(A, nA, B, nB, r1);
-					std::merge(A + i0, A + i1, B + (r0 - i0), B + (r1 - i1), dst + a + r0, name_less);
-				});
-			}
-			for (size_t k = 0; k < pool.size(); ++k) pool[k].join();
-			std::swap(src, dst);
-		}
-		if (src != order.data()) parallel_for(T, n, [&](int, size_t lo, size_t hi) { std::copy(src + lo, src + hi, order.data() + lo); });
-	}
-
-	lap("sort by name");
-	// ---- SoA columns ----
-	const u32 n = (u32) order.size();
+	// ---- the host image of the table (strandedness, fragment length, the event glue and the output read it) ----
+	const u32 n = sz.n_fragments;
+	const size_t n3 = 3 * (size_t) n;
 	out.n = n;
-	// columns are sized without being touched; each thread zeroes and fills its own range (parallel first touch)
 	out.n_aln.resize(n); out.fflags.resize(n); out.filter.resize(n);
-	out.contig.resize(3 * (size_t) n); out.start.resize(3 * (size_t) n); out.end.resize(3 * (size_t) n); out.aflags.resize(3 * (size_t) n);
-	out.cigar_off.resize(3 * (size_t) n); out.cigar_cnt.resize(3 * (size_t) n); out.seq_off.resize(3 * (size_t) n); out.seq_len.resize(3 * (size_t) n);
-	out.genes_off.resize(3 * (size_t) n); out.genes_cnt.resize(3 * (size_t) n);
-	out.name_off.resize((size_t) n + 1);
-	// pool offsets: prefix sums over the fragments in name order (sizes in parallel, scan serial over contiguous arrays)
-	column<u64> cig_at((size_t) n + 1), seq_at((size_t) n + 1);
-	cig_at[0] = seq_at[0] = 0; out.name_off[0] = 0;
-	parallel_for(T, (size_t) n, [&](int, size_t lo, size_t hi) {
-		for (size_t i = lo; i < hi; ++i) {
-			// fragments in name order lie all over the workers' pools: the records of the ones a few steps ahead are requested early
-			if (i + 32 < hi) __builtin_prefetch(&workers[order[i + 32].worker].frags[order[i + 32].frag]);
-			if (i + 16 < hi) { const worker& w8 = workers[order[i + 16].worker]; __builtin_prefetch(&w8.norm_alns[w8.frags[order[i + 16].frag].head]); }
-			const worker& w = workers[order[i].worker]; const frag_build& fb = w.frags[order[i].frag];
-			u64 nc = 0, ns = 0;
-			for (u32 s = 0; s < fb.count; ++s) { const aln_build& a = w.norm_alns[fb.head + s]; nc += a.cigar_cnt; if (s < 2) ns += ((a.seq_len + 1) / 2 + 15) / 16; }
-			cig_at[i + 1] = nc; seq_at[i + 1] = ns; out.name_off[i + 1] = fb.name_len;
-		}
-	});
-	for (u32 i = 0; i < n; ++i) { cig_at[i + 1] += cig_at[i]; seq_at[i + 1] += seq_at[i]; out.name_off[i + 1] += out.name_off[i]; }
-	if (cig_at[n] > 0xFFFFFFFFull || seq_at[n] > 0xFFFFFFFFull) fail("chunk too large: more than 2^32 CIGAR operations or 64 GiB of sequence");
-	out.cigar.resize(cig_at[n] + 1); out.seq.resize(seq_at[n] * 16 + 16); out.names.resize(out.name_off[n]);
-	out.cigar[cig_at[n]] = 0; memset(&out.seq[seq_at[n] * 16], 0, 16);
-	parallel_for(T, (size_t) n, [&](int, size_t lo, size_t hi) {
-		for (size_t i = lo; i < hi; ++i) {
-			if (i + 32 < hi) __builtin_prefetch(&workers[order[i + 32].worker].frags[order[i + 32].frag]);
-			if (i + 16 < hi) {
-				const worker& w8 = workers[order[i + 16].worker]; const frag_build& f8 = w8.frags[order[i + 16].frag];
-				__builtin_prefetch(&w8.norm_alns[f8.head]); __builtin_prefetch(&w8.norm_alns[f8.head] + 2); __builtin_prefetch(w8.names.data() + f8.name_off);
-			}
-			if (i + 8 < hi) {
-				const worker& w4 = workers[order[i + 8].worker]; const frag_build& f4 = w4.frags[order[i + 8].frag];
-				for (u32 s = 0; s < f4.count; ++s) { const aln_build& a = w4.norm_alns[f4.head + s]; __builtin_prefetch(&w4.norm_cigars[a.cigar_off]); if (s < 2 && a.seq_len) { __builtin_prefetch(&w4.seqs[a.seq_off]); __builtin_prefetch(&w4.seqs[a.seq_off] + 48); } }
-			}
-			const worker& w = workers[order[i].worker]; const frag_build& fb = w.frags[order[i].frag];
-			out.n_aln[i] = (u8) fb.count; out.fflags[i] = (fb.single_end ? FF_SINGLE_END : 0) | (fb.duplicate ? FF_DUPLICATE : 0); out.filter[i] = 0;
-			memcpy(&out.names[out.name_off[i]], w.names.data() + fb.name_off, fb.name_len);
-			u64 c = cig_at[i], sq = seq_at[i];
-			if (seq_at[i + 1] > sq) memset(&out.seq[sq * 16], 0, (seq_at[i + 1] - sq) * 16); // padding of the 16-byte units
-			for (u32 s = fb.count; s < 3; ++s) { // unused slot
-				const size_t x = (size_t) s * n + i;
-				out.contig[x] = 0; out.start[x] = 0; out.end[x] = 0; out.aflags[x] = 0; out.cigar_off[x] = 0; out.cigar_cnt[x] = 0; out.seq_off[x] = 0; out.seq_len[x] = 0;
-			}
-			for (u32 s = 0; s < 3; ++s) { const size_t x = (size_t) s * n + i; out.genes_off[x] = 0; out.genes_cnt[x] = 0; if (s == 2) { out.seq_off[x] = 0; out.seq_len[x] = 0; } }
-			for (u32 s = 0; s < fb.count; ++s) {
-				const aln_build& a = w.norm_alns[fb.head + s];
-				const size_t x = (size_t) s * n + i;
-				out.contig[x] = a.contig; out.start[x] = a.start; out.end[x] = a.end;
-				out.aflags[x] = (a.supplementary ? AF_SUPPLEMENTARY : 0) | (a.first_in_pair ? AF_FIRST_IN_PAIR : 0) | (a.forward ? AF_FORWARD : 0) | AF_PRED_AMBIGUOUS;
-				out.cigar_off[x] = (u32) c; out.cigar_cnt[x] = (u16) a.cigar_cnt;
-				memcpy(&out.cigar[c], &w.norm_cigars[a.cigar_off], 4ull * a.cigar_cnt); c += a.cigar_cnt;
-				if (s < 2) {
-					out.seq_off[x] = (u32) sq; out.seq_len[x] = (u16) a.seq_len;
-					if (a.seq_len) memcpy(&out.seq[sq * 16], &w.seqs[a.seq_off], (a.seq_len + 1) / 2);
-					sq += ((a.seq_len + 1) / 2 + 15) / 16;
-				}
-			}
-		}
-	});
-	out.seq_off.resize(2 * (size_t) n); out.seq_len.resize(2 * (size_t) n);
-	lap("SoA columns");
-
-	// ---- multimappers: neighbours in name order that share the name up to the last comma (read_chimeric_alignments.cpp:792-802) ----
-	auto stem_len = [&](u32 i) { const char* s = out.names.data() + out.name_off[i]; u64 l = out.name_off[i + 1] - out.name_off[i]; u64 k = l; while (k > 0 && s[k - 1] != ',') --k; return k > 0 ? k - 1 : l; };
-	{ // pairs (i, i+1) tested on all threads; a fragment is flagged from either side, so the flags are set after the tests (no two threads write one byte)
-		std::vector<u8> same(n, 0);
-		parallel_for(T, n > 0 ? (size_t) n - 1 : 0, [&](int, size_t lo, size_t hi) {
-			for (size_t i = lo; i < hi; ++i) { const u64 la = stem_len((u32) i), lb = stem_len((u32) i + 1); same[i] = la == lb && memcmp(out.names.data() + out.name_off[i], out.names.data() + out.name_off[i + 1], la) == 0; }
-		});
-		parallel_for(T, (size_t) n, [&](int, size_t lo, size_t hi) { for (size_t i = lo; i < hi; ++i) { if (same[i] || (i > 0 && same[i - 1])) out.fflags[i] |= FF_MULTIMAPPER; if (i > 0 && same[i - 1]) out.fflags[i] |= FF_SAME_NAME_AS_PREVIOUS; } });
-	}
+	out.contig.resize(n3); out.start.resize(n3); out.end.resize(n3); out.aflags.resize(n3); out.cigar_off.resize(n3); out.cigar_cnt.resize(n3);
+	out.seq_off.resize(2 * (size_t) n); out.seq_len.resize(2 * (size_t) n); out.genes_off.resize(n3); out.genes_cnt.resize(n3);
+	out.cigar.resize(sz.n_cigar); out.seq.resize(sz.n_seq_bytes); out.names.resize(sz.n_name_bytes); out.name_off.resize((size_t) n + 1);
+	// the gene sets come with the annotation; until then they are empty (zeroed here while the copies run)
+	std::thread zero_genes([&]() { memset(out.genes_off.data(), 0, n3 * sizeof(u32)); memset(out.genes_cnt.data(), 0, n3 * sizeof(u16)); });
+	arb_fragment_columns cols = {out.n_aln.data(), out.fflags.data(), out.filter.data(), out.contig.data(), out.start.data(), out.end.data(), out.aflags.data(), out.cigar_off.data(),
+	                             out.cigar_cnt.data(), out.seq_off.data(), out.seq_len.data(), out.cigar.data(), out.seq.data(), out.names.data(), out.name_off.data()};
+	const int rc = arb_get_fragment_table(opt.scan_ctx, &cols);
+	zero_genes.join();
+	if (rc != 0) fail(arb_last_error(opt.scan_ctx));
 	stats.t_finalize = now_s() - tf;
-	lap("multimapper flags");
+	lap("fragment table -> host");
 	// the workers go back to the cache when `held` leaves scope (their contents are dropped by a helper thread)
 	lap("free worker state");
 }

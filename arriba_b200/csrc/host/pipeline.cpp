@@ -97,23 +97,12 @@ void pipeline::upload_reference() {
 	reference_on_device = true; contigs_on_device = nc;
 }
 
-arb_soa_chunk pipeline::chunk_of(fragment_table& frags) {
-	arb_soa_chunk c;
-	c.n_fragments = frags.n; c.n_aln = frags.n_aln.data(); c.fflags = frags.fflags.data(); c.filter = frags.filter.data();
-	c.contig = frags.contig.data(); c.start = frags.start.data(); c.end = frags.end.data(); c.aflags = frags.aflags.data();
-	c.cigar_off = frags.cigar_off.data(); c.cigar_cnt = frags.cigar_cnt.data(); c.seq_off = frags.seq_off.data(); c.seq_len = frags.seq_len.data();
-	c.genes_off = frags.genes_off.data(); c.genes_cnt = frags.genes_cnt.data();
-	c.cigar = frags.cigar.data(); c.n_cigar = frags.cigar.size(); c.seq = frags.seq.data(); c.n_seq_bytes = frags.seq.size(); c.genes = frags.genes.data(); c.n_genes = frags.genes.size();
-	return c;
-}
-
-// end of ingest: the genome and every column ingest produced start their way to the device while the host annotates (the gene sets follow in upload())
+// end of ingest: the genome follows the fragment table, which ingest left resident on the device (arb_build_fragment_table); the annotation columns
+// follow in annotate()
 void pipeline::begin_upload() {
 	ref.set_contig_flags(opt.interesting_contigs, opt.viral_contigs); // the contig table is complete once the BAM header has been read
 	ref.flatten();
 	upload_reference();
-	arb_soa_chunk c = chunk_of(frags);
-	check(ctx, arb_push_chunk_begin(ctx, &c), "arb_push_chunk_begin");
 	upload_begun = true;
 }
 

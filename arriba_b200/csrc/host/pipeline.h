@@ -57,7 +57,7 @@ struct pipeline {
 	void ingest();
 	void annotate();
 	void upload();
-	void upload_reference(); void send_annotation(); void begin_upload(); arb_soa_chunk chunk_of(fragment_table& t); bool upload_begun; // ingest ends by starting the copy of its columns; annotation overlaps it
+	void upload_reference(); void send_annotation(); void begin_upload(); bool upload_begun; // ingest leaves the fragment table resident; the genome follows before annotation
 	void read_filters();
 	void fragment_length();
 	void find_fusions();

@@ -116,6 +116,33 @@ int arb_push_chunk_end(arb_ctx* ctx, const arb_soa_chunk* chunk);
  * record_offsets: capacity bytes / 36 + 1; malformed != 0: a block_size < 33 was met where a one-thread walk would have met it. */
 int arb_bam_scan(arb_ctx* ctx, const uint8_t* chunk, uint64_t bytes, uint64_t first, int32_t n_ref, uint32_t n_lists, uint64_t* consumed, uint32_t* n_records,
                  uint32_t* list_begin /* n_lists + 1 */, uint32_t* record_offsets, uint32_t* malformed);
+/* ---- the fragment table, built on the device from the ingest workers' pools ---------------------------------------
+ * The end of read_chimeric_alignments (source/read_chimeric_alignments.cpp:340-506 slot normalisation and rejection of malformed fragments, the std::map
+ * order of "<qname>,<HI>[ITD]", :792-802 mark_multimappers). Every worker of the record loop owns append-only pools: read names, CIGAR operations, nt16
+ * sequences (each 16-byte aligned), alignments (linked per fragment through `next`, worker-local indices) and fragments (`head` = first alignment; offsets
+ * into the worker's own pools). arb_build_fragment_table copies the pools to the device and leaves the fragment table resident in name order, as
+ * arb_push_chunk_begin would (the annotation columns follow through arb_annotate_pass1/2). arb_get_fragment_table copies it back into caller columns sized
+ * from `sizes`: 3*n per slot column (seq_off / seq_len 2*n), n_cigar, n_seq_bytes, n_name_bytes, n + 1 name offsets. Names of one table must be unique. */
+typedef struct arb_pool_alignment { uint8_t supplementary, first_in_pair, forward; uint16_t contig; int32_t start, end; uint32_t cigar_off, cigar_cnt; uint64_t seq_off; uint32_t seq_len; int32_t next; } arb_pool_alignment;
+typedef struct arb_pool_fragment { uint64_t name_off; uint32_t name_len; int32_t head, tail; uint32_t count; uint8_t single_end, duplicate; } arb_pool_fragment;
+typedef struct arb_ingest_pool {
+	const char* names; uint64_t n_name_bytes; const uint32_t* cigars; uint64_t n_cigars; const uint8_t* seqs; uint64_t n_seq_bytes;
+	const arb_pool_alignment* alns; uint64_t n_alns; const arb_pool_fragment* frags; uint32_t n_frags;
+} arb_ingest_pool;
+typedef struct arb_fragment_table_sizes {
+	uint32_t n_fragments;  /* fragments that survived slot normalisation */
+	uint32_t tie_rounds;   /* rounds of the name sort beyond the first 16 bytes of the names */
+	uint64_t n_rejected;   /* malformed fragments (the reference's "malformed SAM records" warning counts them) */
+	uint64_t n_cigar, n_seq_bytes, n_name_bytes;
+	float upload_ms, build_ms;  /* copy of the pools; the whole call (copy included), both on the context's stream */
+} arb_fragment_table_sizes;
+typedef struct arb_fragment_columns {
+	uint8_t* n_aln; uint8_t* fflags; uint8_t* filter; uint16_t* contig; int32_t* start; int32_t* end; uint8_t* aflags; uint32_t* cigar_off; uint16_t* cigar_cnt;
+	uint32_t* seq_off; uint16_t* seq_len; uint32_t* cigar; uint8_t* seq; char* names; uint64_t* name_off;
+} arb_fragment_columns;
+int arb_build_fragment_table(arb_ctx* ctx, const arb_ingest_pool* pools, uint32_t n_pools, arb_fragment_table_sizes* sizes);
+int arb_get_fragment_table(arb_ctx* ctx, const arb_fragment_columns* out);
+uint32_t arb_fragment_table_tie_rounds(arb_ctx* ctx); /* tie_rounds of the last arb_build_fragment_table */
 /* ---- annotation of the resident fragments -------------------------------------------------------------------
  * Replaces the annotation passes of main (source/arriba.cpp:165-325: annotate_alignments per fragment, source/annotation.cpp:431-555; dummy genes for
  * intergenic breakpoints, arriba.cpp:207-260; second pass :262-319) and assign_strands_from_strandedness (source/read_chimeric_alignments.cpp:775-790).
